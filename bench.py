@@ -84,6 +84,11 @@ def make_config(args, cfg, world, lines=True, ring=None, nsets=None, B=None):
     return c
 
 
+def n_input_sets(B, W, H):
+    """Distinct input batches the steps cycle through: more than 126 MB in all, so that inputs are never L2-resident."""
+    return max(2, int(np.ceil(160e6 / (B * W * H))))
+
+
 def gen_frames(cfg, rank, nsets, B=None):
     """nsets distinct input batches (so that the inputs cycle through more than the 126 MB L2)."""
     import synth
@@ -218,6 +223,38 @@ def run_reference(args, cfg):
 
 
 # ------------------------------------------------------------------------------------------------
+DUMP_BYTES = 64 * 10**6
+
+
+def last_step_outputs(pkg, dev_read, B, orb, match, nmatch, lines):
+    """--dump-outputs: what a caller of the timed path receives for one step, as float32 (float64: line equations, counts, frame
+    indices).  A fixed seeded sample of the step's frames f >= 1, as many as DUMP_BYTES holds at full capacity (so the sample depends on
+    the arguments only); for each f its keypoints, descriptors and lines (rows of all sampled frames concatenated, with the counts) and
+    the whole match-table rows of the pair (f - 1, f) (-1 = no match)."""
+    kps, desc, n, cap = orb
+    capl = lines[4] if lines else 0
+    per_frame = cap * (7 + 32 + 1) * 4 + capl * ((17 + 32 + 1) * 4 + 3 * 8) + 6 * 8
+    S = min(B - 1, DUMP_BYTES // per_frame)
+    sel = np.sort(np.random.default_rng(0).choice(np.arange(1, B), S, replace=False))
+    rows = lambda a, cnt: np.concatenate([a[i, :c] for i, c in enumerate(cnt)])
+    fields = lambda a: np.stack([a[f].astype(np.float32) for f in a.dtype.names], -1)
+    n = dev_read(n, np.int32, (B,))[sel]
+    out = {"frames": sel.astype(np.float64), "keypoint_counts": n.astype(np.float64),
+           "keypoints": fields(rows(dev_read(kps, pkg.KEYPOINT_DTYPE, (B, cap))[sel], n)),
+           "descriptors": rows(dev_read(desc, np.uint8, (B, cap, 32))[sel], n).astype(np.float32),
+           "point_matches": match.cpu().numpy()[sel - 1].astype(np.float32), "point_match_counts": nmatch.cpu().numpy()[sel - 1].astype(np.float64)}
+    if lines:
+        kl, ld, eq, nl, capl, lmatch, nlmatch = lines
+        nl = dev_read(nl, np.int32, (B,))[sel]
+        out.update(line_counts=nl.astype(np.float64),
+                   keylines=fields(rows(dev_read(kl, pkg.KEYLINE_DTYPE, (B, capl))[sel], nl)),
+                   line_descriptors=rows(dev_read(ld, np.uint8, (B, capl, 32))[sel], nl).astype(np.float32),
+                   line_equations=rows(dev_read(eq, np.float64, (B, capl, 3))[sel], nl),
+                   line_matches=lmatch.reshape(-1)[:(B - 1) * capl].view(B - 1, capl).cpu().numpy()[sel - 1].astype(np.float32),
+                   line_match_counts=nlmatch.cpu().numpy()[sel - 1].astype(np.float64))
+    return out
+
+
 class ClockSampler:
     def __init__(self, device_index):
         self.idx = device_index; self.samples = []; self.proc = None
@@ -269,6 +306,8 @@ def main():
     ap.add_argument("--no-lines", action="store_true", help="ORB + point matching only")
     ap.add_argument("--line-ring", type=int, default=10, help="line / frame handles (streams + workspaces) kept in flight (measured: 10 gives the shortest step, device-resident and end to end; 6, 8, 12, 14 are 1-2 ms slower)")
     ap.add_argument("--walkers-per-sm", type=float, default=0.0, help="per line handle: resident LSD region walkers per SM (0 = one per frame)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed on rank 0 (a fixed sample of its frames, "
+                    "at most 64 MB) to DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     cfg = WORKLOADS[args.workload]
@@ -324,7 +363,7 @@ def main():
     cap = ext.cap
     voc = synth.vocabulary(NWORDS)
     d_voc = torch.from_numpy(voc).to(dev)
-    nsets = max(2, int(np.ceil(160e6 / (B * W * H))))   # cycle > 126 MB of distinct inputs => inputs never L2-resident
+    nsets = n_input_sets(B, W, H)
     sets = gen_frames(cfg, rank, nsets, B)
     d_sets = [torch.from_numpy(s).to(dev) for s in sets]
     d_match = torch.empty((Bf, cap), dtype=torch.int32, device=dev)
@@ -333,14 +372,17 @@ def main():
     d_nlmatch = [torch.zeros((Bf,), dtype=torch.int32, device=dev) for _ in range(R)]
     d_gather = torch.empty((world * Bf, cap), dtype=torch.int32, device=dev) if world > 1 else None
     d_lgather = torch.empty((world * Bf, NL), dtype=torch.int32, device=dev) if world > 1 else None
-    class _DevArr:                                      # a torch view of a device array owned by the library (counts only)
-        def __init__(self, ptr, n):
-            self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<i4", "data": (ptr, False), "version": 2}
+    class _DevArr:                                      # a torch view of a device array owned by the library
+        def __init__(self, ptr, n, typestr="<i4"):
+            self.__cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (ptr, False), "version": 2}
     _views = {}
     def dev_i32(ptr, n):                                # (the result arrays exist after the handle's first call: looked up per step, cached)
         if (ptr, n) not in _views:
             _views[(ptr, n)] = torch.as_tensor(_DevArr(int(ptr), n), device=dev)
         return _views[(ptr, n)]
+    def dev_read(ptr, dtype, shape):                    # host copy of a device array owned by the library
+        nbytes = int(np.prod(shape)) * np.dtype(dtype).itemsize
+        return torch.as_tensor(_DevArr(int(ptr), nbytes, "|u1"), device=dev).cpu().numpy().view(dtype).reshape(shape)
     u_pts = torch.zeros((), dtype=torch.int64, device=dev)     # features + matches of the timed loop, summed ON the device,
     u_lin = [torch.zeros((), dtype=torch.int64, device=dev) for _ in range(R)]   # inside the timed region (no separate counting pass)
     pending = [False] * R
@@ -439,6 +481,11 @@ def main():
     for l in lsr:
         l.sync()
     launches = launches_now() - launches0
+    dumped = None                                       # read back now: the passes below reuse the handles' result buffers
+    if args.dump_outputs and rank == 0:
+        r = (args.warmup + args.steps - 1) % R if LINES else 0
+        dumped = last_step_outputs(pkg, dev_read, B, ext.device_results(), d_match, d_nmatch,
+                                   lsr[r].device_results() + (d_lmatch[r], d_nlmatch[r]) if LINES else None)
     clocks = sampler.stop() if rank == 0 else None
     units_timed = int(u_pts.item()) + sum(int(u.item()) for u in u_lin)      # counted inside the timed region, on the device
 
@@ -731,8 +778,16 @@ def main():
                         "ms_per_step": e2e_ms / args.steps},
                 "gpu_launches": int(launches), "clocks": clocks, "roofline": roofline, "cpu_baseline": cpu, "cpu_baseline_cv2": cpu_cv2,
                 "gather_check": gather_check, "table_check": table_check, "in_pipeline": in_pipeline}
+        if dumped:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line)); sys.stdout.flush()
-    # orderly teardown: the matchers run on the frame handles' streams, so they go first
+    # orderly teardown.  The pinned match tables were copied into on the frame handles' streams, and torch records an event on every such
+    # stream when it frees a pinned block: they are freed while those streams exist.  The matchers run on the frame handles' streams, so
+    # they are closed before the frames.
+    torch.cuda.synchronize()
+    del h_match, h_nmatch, h_lmatch, h_nlmatch
     torch.cuda.synchronize()
     for m_ in mts + lms:
         m_.close()
@@ -740,14 +795,9 @@ def main():
         f_.close()
     if world > 1:
         dist.destroy_process_group()
-    # leave here: the tensors of this frame alias device memory of the handles closed above, and their destructors (run on return)
-    # were seen to fault inside torch at interpreter exit; everything has been printed, synchronised and closed in order
-    sys.stdout.flush(); sys.stderr.flush()
-    os._exit(0)
+    return 0
 
 
 if __name__ == "__main__":
     import faulthandler; faulthandler.enable()
-    rc = main()
-    sys.stdout.flush(); sys.stderr.flush()
-    os._exit(rc)          # handles are closed in order above; skip interpreter-exit destructors (arbitrary order across CUDA objects)
+    sys.exit(main())

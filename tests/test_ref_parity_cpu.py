@@ -1,25 +1,29 @@
 """The oracle's restatement (oracle/*.cpp) held against THE REFERENCE ITSELF: oracle/_ref/libref.so is the reference's own
 src/ORBextractor.cc, ORBmatcher.cc, LSDmatcher.cpp, ExtractLineSegment.cpp, Frame.cc, KeyFrame.cc, MapPoint.cc, MapLine.cpp and
-Thirdparty/DBoW2, compiled unmodified by oracle/ref_build.sh (needs /root/reference: this container; elsewhere the prebuilt
-library is used, and the committed fixtures of tests/golden/ref_*.npz carry the same outputs — tests/test_ref_golden_cpu.py).
+Thirdparty/DBoW2, compiled unmodified by oracle/ref_build.sh.  What those calls returned is recorded in tests/golden/ref_parity.npz
+(tests/ref_replay.py), so the comparisons run without the reference's sources.
 
 Bit-exact everywhere (ints, bytes, indices, and the f32 keypoint fields)."""
 import os
 import numpy as np
 import pytest
 
+import ref_replay
+
 
 @pytest.fixture(scope="module")
-def ref():
-    from oracle import ref as R
-    if not R.available():
-        pytest.skip("oracle/_ref/libref.so not built and /root/reference absent")
-    R.lib()
-    return R
+def ref_store():
+    store = ref_replay.Store()
+    yield store
+    store.save()
 
 
-def _same_kps(a, b):
-    return len(a) == len(b) and a.tobytes() == b.tobytes()
+@pytest.fixture
+def ref(ref_store, request):
+    return ref_store.reference(request.node.name)
+
+
+_same = ref_replay.same
 
 
 # ---------------------------------------------------------------------------------------------- ORB extractor
@@ -41,16 +45,17 @@ def test_orb_icl_frame_known_answers(oracle, ref, icl_gray):
     import hashlib
     k, d, lc = ref.orb_extract(icl_gray, 1000)
     assert list(lc) == [218, 181, 151, 126, 105, 88, 73, 60] and len(k) == 1002
-    assert hashlib.sha1(d.tobytes()).hexdigest() == "e8dce82582b67285476bbe582e3557644739a438"
-    uva = np.stack([k["x"], k["y"], k["angle"]], 1).astype(np.float32)
-    assert hashlib.sha1(uva.tobytes()).hexdigest() == "1105debd69ac4a65f0375a9da3f130fe9fd64ca5"
-    assert list(d[0]) == [176, 12, 22, 27, 144, 163, 2, 87, 84, 11, 99, 80, 66, 49, 32, 65, 81, 2, 2, 34, 49, 184, 81, 31, 36, 174, 48, 64, 72, 64, 224, 137]
     ok, od = oracle.OrbOracle(1000, 1.2, 8, 20, 7).extract(icl_gray)
-    assert _same_kps(k, ok) and np.array_equal(d, od)
+    assert _same(k, ok) and _same(d, od)
+    # (the known answers, on the oracle's output: equal to the reference's above)
+    assert hashlib.sha1(od.tobytes()).hexdigest() == "e8dce82582b67285476bbe582e3557644739a438"
+    uva = np.stack([ok["x"], ok["y"], ok["angle"]], 1).astype(np.float32)
+    assert hashlib.sha1(uva.tobytes()).hexdigest() == "1105debd69ac4a65f0375a9da3f130fe9fd64ca5"
+    assert list(od[0]) == [176, 12, 22, 27, 144, 163, 2, 87, 84, 11, 99, 80, 66, 49, 32, 65, 81, 2, 2, 34, 49, 184, 81, 31, 36, 174, 48, 64, 72, 64, 224, 137]
     # the initialiser extractor (2 * nFeatures, Tracking.cc:120)
     k2, d2, _ = ref.orb_extract(icl_gray, 2000)
     ok2, od2 = oracle.OrbOracle(2000, 1.2, 8, 20, 7).extract(icl_gray)
-    assert _same_kps(k2, ok2) and np.array_equal(d2, od2)
+    assert _same(k2, ok2) and _same(d2, od2)
 
 
 @pytest.mark.parametrize("f", range(8))
@@ -58,27 +63,27 @@ def test_orb_synthetic_640(oracle, ref, synth, f):
     img = synth.frame(640, 480, f * 5)
     k, d, _ = ref.orb_extract(img, 1000)
     ok, od = oracle.OrbOracle(1000, 1.2, 8, 20, 7).extract(img)
-    assert _same_kps(k, ok) and np.array_equal(d, od) and len(k) > 900
+    assert _same(k, ok) and _same(d, od) and len(k) > 900
 
 
 def test_orb_1280_4000_and_other_parameters(oracle, ref, synth):
     img = synth.frame(1280, 960, 3)
     k, d, _ = ref.orb_extract(img, 4000)
     ok, od = oracle.OrbOracle(4000, 1.2, 8, 20, 7).extract(img)
-    assert _same_kps(k, ok) and np.array_equal(d, od) and len(k) > 3900
+    assert _same(k, ok) and _same(d, od) and len(k) > 3900
     small = synth.frame(640, 480, 2)[:241, :323]
     for nf, sc, nl, ini, mn in [(500, 1.5, 4, 30, 10), (300, 1.2, 8, 20, 7), (1500, 1.1, 6, 12, 5)]:
         k, d, _ = ref.orb_extract(small, nf, sc, nl, ini, mn)
         ok, od = oracle.OrbOracle(nf, sc, nl, ini, mn).extract(small)
-        assert _same_kps(k, ok) and np.array_equal(d, od), (nf, sc, nl)
+        assert _same(k, ok) and _same(d, od), (nf, sc, nl)
 
 
 def test_pyramid_levels(oracle, ref, icl_gray):
     """ComputePyramid (ORBextractor.cc:1107-1132): every level and its 19-px bordered view."""
     orc = oracle.OrbOracle(1000, 1.2, 8, 20, 7); orc.extract(icl_gray)
     for l in range(8):
-        assert np.array_equal(ref.orb_pyramid_level(icl_gray, l, False), orc.level(l, False)), l
-        assert np.array_equal(ref.orb_pyramid_level(icl_gray, l, True), orc.level(l, True)), l
+        assert _same(ref.orb_pyramid_level(icl_gray, l, False), orc.level(l, False)), l
+        assert _same(ref.orb_pyramid_level(icl_gray, l, True), orc.level(l, True)), l
 
 
 def test_octree_tie_rule(oracle, ref):
@@ -96,7 +101,7 @@ def test_octree_tie_rule(oracle, ref):
         N = int(rng.integers(1, 400))
         got = ref.octree(xs, ys, resp, 0, W, 0, H, N)
         exp = oracle.octree(xs, ys, resp, 0, W, 0, H, N)
-        assert np.array_equal(got, exp), trial
+        assert _same(got, exp), trial
 
 
 # ---------------------------------------------------------------------------------------------- point matchers
@@ -131,12 +136,12 @@ def test_search_by_bow(oracle, ref, synth, nwords, mask, ratio, ori, f0):
     # the reference skips BAD MapPoints exactly like missing ones (:197-200): make a third of the invalid ones bad instead of NULL
     state1 = valid1.copy(); inv = np.flatnonzero(valid1 == 0); state1[inv[::3]] = 2
     n_r, m_r = ref.search_by_bow(d1, k1, d2, k2, fv1, fv2, state1, ratio, ori)
-    assert n_r == n_o and np.array_equal(m_r, m_o)
+    assert n_r == n_o and _same(m_r, m_o)
     valid2 = (rng.random(len(d2)) < 0.8).astype(np.uint8)
     n_o, m_o = oracle.search_by_bow_kf(d1, d2, fv1, fv2, valid1, valid2, k1["angle"], k2["angle"], ratio, ori)
     state2 = valid2.copy(); inv = np.flatnonzero(valid2 == 0); state2[inv[::2]] = 2
     n_r, m_r = ref.search_by_bow_kf(d1, k1, d2, k2, fv1, fv2, state1, state2, ratio, ori)
-    assert n_r == n_o and np.array_equal(m_r, m_o)
+    assert n_r == n_o and _same(m_r, m_o)
     assert n_o > 10 or nwords == 1000
 
 
@@ -148,7 +153,7 @@ def test_search_by_bow_icl_shifted(oracle, ref, icl_gray, synth):
     v = np.ones(len(d1), np.uint8)
     n_o, m_o = oracle.search_by_bow(d1, d2, fv1, fv2, v, k1["angle"], k2["angle"], 0.7, True)
     n_r, m_r = ref.search_by_bow(d1, k1, d2, k2, fv1, fv2, v, 0.7, True)
-    assert n_r == n_o and np.array_equal(m_r, m_o) and n_o > 300
+    assert n_r == n_o and _same(m_r, m_o) and n_o > 300
 
 
 def _poses(rng, epi_inside):
@@ -178,7 +183,7 @@ def test_search_for_triangulation(oracle, ref, synth, nwords, ori, inside, f0):
     n_r, p_r, (ex, ey) = ref.search_for_triangulation(d1, k1, d2, k2, fv1, fv2, has1, has2, ref.CAM640, T1, T2, F12, ori)
     tb = orc.tables(); scale, sigma2 = tb["scale"], tb["sigma2"]
     n_o, p_o = oracle.search_for_triangulation(d1, d2, fv1, fv2, has1, has2, k1, k2, F12, ex, ey, scale, sigma2, ori)
-    assert n_r == n_o and np.array_equal(p_r, p_o)
+    assert n_r == n_o and _same(p_r, p_o)
     assert (0 <= ex < 640 and 0 <= ey < 480) == inside
 
 
@@ -192,7 +197,7 @@ def test_features_in_area(oracle, ref, synth):
         lo, hi = (-1, -1) if rng.random() < 0.3 else (int(rng.integers(0, 5)), int(rng.integers(0, 8)))
         got = ref.features_in_area(k1, camv, x, y, r, lo, hi)
         exp = oracle.features_in_area(k1["x"], k1["y"], k1["octave"], (0, 640, 0, 480), x, y, r, lo, hi)
-        assert np.array_equal(got, exp)
+        assert _same(got, exp)
 
 
 @pytest.mark.parametrize("seed,th,mono,ori,claimed", [(1, 15.0, True, True, 0.05), (2, 7.0, True, True, 0.0), (3, 30.0, True, False, 0.2),
@@ -248,12 +253,12 @@ def test_search_for_initialization(oracle, ref, synth, f0, window, ratio, ori, n
     bounds = (0.0, 640.0, 0.0, 480.0)
     n_o, m_o, p_o = oracle.search_for_initialization(d1, k1, d2, k2, prev, bounds, ratio, ori, window)
     n_r, m_r, p_r = ref.search_for_initialization(d1, k1, d2, k2, prev, ref.cam(500, 500, 320, 240, *bounds), 8, 1.2, ratio, ori, window)
-    assert n_r == n_o and np.array_equal(m_r, m_o) and np.array_equal(p_r, p_o)
+    assert n_r == n_o and _same(m_r, m_o) and _same(p_r, p_o)
     assert n_o > 50 or window < 20
     # second call, as Tracking does on the next frame with the updated vbPrevMatched
     n_o2, m_o2, _ = oracle.search_for_initialization(d1, k1, d2, k2, p_o, bounds, ratio, ori, window)
     n_r2, m_r2, _ = ref.search_for_initialization(d1, k1, d2, k2, p_r, ref.cam(500, 500, 320, 240, *bounds), 8, 1.2, ratio, ori, window)
-    assert n_r2 == n_o2 and np.array_equal(m_r2, m_o2)
+    assert n_r2 == n_o2 and _same(m_r2, m_o2)
 
 
 def test_descriptor_medoid(oracle, ref):
@@ -287,11 +292,11 @@ def test_line_matchers(oracle, ref, n1, n2, seed):
     for mode in (0, 1, 2, 3):
         n_o, m_o = oracle.line_match(mode, d1, d2, h1, h2)
         n_r, m_r, mad = ref.line_match(mode, d1, d2, h1, h2)
-        assert n_r == n_o and np.array_equal(m_r, m_o), mode
+        assert n_r == n_o and _same(m_r, m_o), mode
         assert mad == oracle.line_mad(knn)
     n_r, m_r, _ = ref.line_match(4, d1, d2, h1, h2)          # SearchByDescriptor(KF, F) has the body of SearchByProjection(KF, F)
     n_o, m_o = oracle.line_match(0, d1, d2, h1, h2)
-    assert n_r == n_o and np.array_equal(m_r, m_o)
+    assert n_r == n_o and _same(m_r, m_o)
 
 
 # ---------------------------------------------------------------------------------------------- DBoW2
@@ -334,7 +339,7 @@ def test_dbow2_transform(oracle, ref, pkg, synth, tmp_path, k, L, stop, early):
     for levelsup in (4, 1, 0, 10):
         node_r, ids_r, w_r = voc.transform(feats, levelsup)
         word_o, node_o, w_o = oracle.vocab_transform(L, parent, nd2, w, leaf, feats, levelsup)
-        assert np.array_equal(word_r, word_o) and np.array_equal(wt_r, w_o)
+        assert _same(word_r, word_o) and _same(wt_r, w_o)
         # stopped words are left out (:1162-1166).  A leaf that sits ABOVE level L - levelsup never assigns *nid (:1254): the
         # reference then files the feature under an indeterminate node (the caller's `NodeId nid` is uninitialised, :1150); the
         # oracle and the kernel file it under the root.  Real vocabularies (ORBvoc: k=10, L=6, levelsup=4) have no such leaves.
@@ -344,7 +349,7 @@ def test_dbow2_transform(oracle, ref, pkg, synth, tmp_path, k, L, stop, early):
         assert np.all(node_o[~defined] == 0)
         node_o = np.where(defined, node_o, node_r)                # (compare the assemblies on the reference's filing)
         ids_p, vals_p = V.bow_vector(word_o, w_o)
-        assert np.array_equal(ids_r, ids_p) and np.array_equal(w_r, vals_p)
+        assert _same(ids_r, ids_p) and _same(w_r, vals_p)
         nodes_p, off_p, idx_p = pkg.Vocabulary.feature_vector(node_o, w_o)
         for j, nid in enumerate(nodes_p):
             assert np.array_equal(np.flatnonzero(node_r == nid), idx_p[off_p[j]:off_p[j + 1]])
@@ -371,9 +376,9 @@ def test_frame_constructor(oracle, ref, icl_gray):
     """Frame::Frame(imGray, ...) (Frame.cc:69-131): ExtractORB + ExtractLSD + UndistortKeyPoints + AssignFeaturesToGrid."""
     fr = ref.frame_from_image(icl_gray)
     ok, od = oracle.OrbOracle(1000, 1.2, 8, 20, 7).extract(icl_gray)
-    assert _same_kps(fr["keys"], ok) and _same_kps(fr["keysUn"], ok) and np.array_equal(fr["desc"], od)
+    assert _same(fr["keys"], ok) and _same(fr["keysUn"], ok) and _same(fr["desc"], od)
     okl, old, oeq = oracle.LineOracle(40).extract(icl_gray)
-    assert fr["keylines"].tobytes() == okl.tobytes() and np.array_equal(fr["ldesc"], old) and np.array_equal(fr["lineeq"], oeq)
+    assert _same(fr["keylines"], okl) and _same(fr["ldesc"], old) and _same(fr["lineeq"], oeq)
     assert list(fr["bounds"]) == [0, 640, 0, 480]
     # grid cell (c, r) holds the features whose rounded cell is (c, r), ascending
     rnd = lambda v: np.floor(v.astype(np.float32) + np.float32(0.5)).astype(int)      # C round() on non-negative floats (PosInGrid, Frame.cc:462-472)
