@@ -42,22 +42,19 @@ struct LineGeom {
     int min_reg_size;
     int trace_cap;              // rows of the debug trace per frame (0 = off)
     int dbg;                    // SSLPL_WALKER_DBG bit mask (bring-up switches of the region walker)
-    int dbg_seed;               // SSLPL_WALKER_SEED: pixel index whose first region list is printed (bring-up)
 };
 
 // What region growing reads per neighbour, in one 16-byte load: level-line angle (degrees, NOTDEF_F when undefined),
 // (float)cos / sin of (float)(angle in radians) — the values region_grow sums — and the mutable `used` flag.
-struct __align__(16) LPix { float ang, cx, cy; unsigned used; };   // `used` = ticket of the region-growing attempt holding the pixel (0 = none)
+// `used`: 0 = free.  The multi-warp walker stores the ticket of the region-growing attempt holding the pixel, the one-warp walker 1.
+struct __align__(16) LPix { float ang, cx, cy; unsigned used; };
 
 struct LineWs {
     uint8_t* blur7; uint8_t* blur5; uint8_t* scaled;
     float* angdeg; LPix* pix; float2* cs0; double* modgrad;
     unsigned long long* maxgrad; unsigned* seeds; int* nseeds;
     unsigned* reg;              // region pixel list (x | y << 16) of the turn holder (whole-frame capacity)
-    unsigned* sreg;             // per frame: WALK_RING speculation slots x WALK_SLOT_CAP list entries (v3: one list of V3_LIST entries per worker)
-    unsigned* dlist;            // v3, per frame: V3_DPOOL entries (see V3Shared::dl_off)
-    unsigned char* rcode;       // v3, per frame: one byte per rank: the try it committed with | 0x80 if it released pixels, 0xff = none
-    double* sjob;               // per frame: one pending NFA job (13 doubles) per speculation slot
+    unsigned* sreg;             // per frame: WALK_RING speculation slots x WALK_SLOT_CAP list entries
     unsigned long long* wstat;  // walker statistics (whole launch): see sslpl_line_walker_stats
     double* seg;                // raw rectangles: x1,y1,x2,y2 (detection scale, before +0.5)
     int* nseg;
@@ -350,7 +347,6 @@ struct WalkCtx {                // context of one walker warp (k_lsd_regions): s
     int abort;                  // speculative attempt abandoned: 1 = capacity, 2 = a live attempt of LOWER rank holds a pixel it needs
     int conflict;               // abort == 2: that rank (the attempt can be repeated once it has been retired)
     unsigned ticket;
-    int dirty, ndeps; unsigned dep[2];   // v3: released pixels; tickets of live lower attempts whose pixels were assumed used
 };
 struct FrameCtl {               // one per walker CTA
     unsigned cursor, nclaims, turn;
@@ -366,10 +362,9 @@ __shared__ __align__(16) double s_stc[WALK_MAXW][96];     // per warp: staging o
 __shared__ WalkCtx s_W1;                                   // the one-warp throughput kernel keeps its own small context:
 __shared__ __align__(16) double s_st1[96];                 // 28 of its CTAs share an SM
 constexpr int SOLO = 0;                                    // (hidden by the template parameter of the same name inside the helpers)
-// SOLO: 0 = multi-warp walker of round 2a (k_lsd_regions), 1 / 2 = one warp per frame (round-2a form / lean), 3 = multi-warp walker v3,
-// 4 = lane-parallel walker (one warp per frame; the cooperative routines work on the region of one lane)
-#define s_W (*((SOLO == 1 || SOLO == 2 || SOLO == 4) ? &s_W1 : &s_Wc[threadIdx.x >> 5]))
-#define s_st ((SOLO == 1 || SOLO == 2 || SOLO == 4) ? s_st1 : s_stc[threadIdx.x >> 5])
+// SOLO: 0 = multi-warp walker (k_lsd_regions), 1 = one warp per frame (k_lsd_regions_solo)
+#define s_W (*(SOLO == 1 ? &s_W1 : &s_Wc[threadIdx.x >> 5]))
+#define s_st (SOLO == 1 ? s_st1 : s_stc[threadIdx.x >> 5])
 
 // SLOT_PRESUMED: the seed was under the ticket of a live attempt of lower rank when its turn to be grown came: it is presumed
 // swallowed; the commit checks (and grows it for real if it was not).  SLOT_ABORTED: to be redone by the turn holder.
@@ -380,11 +375,8 @@ __device__ __forceinline__ unsigned l_turn() { return *reinterpret_cast<volatile
 __device__ __forceinline__ bool l_bit(const unsigned* bits, int q) { return (reinterpret_cast<const volatile unsigned*>(bits)[q >> 5] >> (q & 31)) & 1u; }
 // Is ticket m (not mine) held by an attempt that has not been retired yet?  Ranks below `turn` are committed or discarded.
 __device__ __forceinline__ bool l_live(unsigned m, int* seq_out) { const int s = (int)(m & 0xffffffu) - 1; *seq_out = s; return m != 0u && s >= (int)l_turn(); }
-// (v3: a released pixel keeps the ticket with bit 31 set: it is free for everybody, but an attempt of LOWER rank that takes it still
-//  poisons the releasing attempt, whose first growth went over a pixel that the sequential order gives to the lower rank)
 template <int SOLO> __device__ __forceinline__ void l_release(const WalkCtx& W, int q) {
-    if (SOLO == 1 || SOLO == 2) W.pix[q].used = 0u;
-    else if (SOLO == 3 || SOLO == 4) atomicCAS(&W.pix[q].used, W.ticket, W.ticket | 0x80000000u);
+    if (SOLO == 1) W.pix[q].used = 0u;
     else atomicCAS(&W.pix[q].used, W.ticket, 0u);
 }
 
@@ -576,116 +568,6 @@ template <int SOLO> __device__ __noinline__ int l_region_grow(int sx, int sy, do
     return n;
 }
 
-
-// -------------------------------------------------------------------------------------------------
-// region_grow, LEAN form (one warp per frame, round 2b).  Same sequential semantics as l_region_grow<1>, restructured around
-// the measured dependent-chain latencies of sm_100a (tools/lat_probe.cu: SHFL 37, MATCH 72, FDIV 57, double alignment test 82,
-// L1 hit 50, L2 hit 280, LDS 34 cycles), because the walker is one warp following one chain:
-//   * the region list's tail lives in a shared-memory ring (the frontier is read with LDS, not through L1/L2; the full list
-//     still goes to global memory for region2rect / refine, fire and forget);
-//   * the alignment test runs on the float DEGREES that both operands come from (|theta - a| <= prec is decided in float
-//     when it is further than 2e-3 deg from the threshold or from the 270-degree fold; closer than that the reference's
-//     double formula decides) — no FP64 and no conversions on the chain;
-//   * the region angle is LAZY: a round tests every pending lane against the exact current angle; the first passing lane k0
-//     is accepted (exact), and every later lane whose outcome cannot change while at most K = popc(passing) more unit
-//     vectors are added to the sums is decided in the same round without recomputing the angle.  The bound is rigorous:
-//     the scan reaches lane l after accepting at most K_l = (first holders among the passing lanes before l) unit vectors, each
-//     within prec + E of S, so S has turned by at most atan(sum |sin phi_i| / |S|) <= 57.3 deg * sin(prec + E) * K_l / |S|;
-//     cv::fastAtan2 is within E = 0.00956 deg of atan2 (measured over 5e8 inputs; 2E = 0.0202 used), float rounding of the
-//     sums is < 3e-4 deg, the rest of the 0.0215 deg is slack.  tools/sim_lean_grow.cpp runs this lane by lane against the
-//     oracle's sequential region_grow (every call of four frames identical).
-//     The round stops before the first lane that is not robust in that sense; only then is the angle recomputed on the
-//     chain.  For big regions (|S| ~ n) nearly every step is ONE round with no atan2 before the next step's loads;
-//   * the angle of the next step is recomputed after that step's loads have been issued (it overlaps their latency);
-//   * duplicates (the same pixel seen from two queue entries) come from one MATCH issued under the record load;
-//   * accepted pixels warm L1 with the six sectors of their 3x3 neighbourhood (consumed one step later).
-// -------------------------------------------------------------------------------------------------
-__device__ int l_region_grow_v3(int sx, int sy, double prec, double* reg_angle_out);
-constexpr int LEAN_RING = 1024;
-__shared__ unsigned s_ring1[LEAN_RING];
-
-__device__ __noinline__ int l_region_grow_lean(int sx, int sy, double prec, double* reg_angle_out) {
-    WalkCtx& W = s_W1;
-    const int lane = threadIdx.x & 31, w = W.w, h = W.h;
-    LPix* pix = W.pix; unsigned* reg = W.reg;
-    const int sq = sy * w + sx;
-    if (lane == 0) { const unsigned pk0 = (unsigned)sx | ((unsigned)sy << 16); reg[0] = pk0; s_ring1[0] = pk0; pix[sq].used = 1u; }
-    float th = __ldg(W.ang + sq);                                // degrees; the region angle is (double)th * L_DEG throughout
-    const float2 c0 = __ldg(W.cs0 + sq);
-    float sumdx = c0.x, sumdy = c0.y;
-    float rM = rsqrtf(sumdx * sumdx + sumdy * sumdy);
-    bool dirty = false;                                          // th / rM are older than the sums
-    int n = 1;
-    const float pdeg = (float)(prec * (180.0 / L_PI));
-    const float coef = (float)(57.2958 * 1.0002 * sin(prec + 0.0006));     // degrees the sums can turn per (accepted vector / |S|): see above
-    const bool rob_ok = prec < 0.78;                             // <= 45 deg: then prec + B <= 75.2 deg < 90 and the reference's fold at 270 deg is the circular distance
-    const int slot = lane >> 3, nb = (lane & 7) + ((lane & 7) >= 4 ? 1 : 0);
-    const int ox = nb % 3 - 1, oy = nb / 3 - 1;
-    const unsigned lt = (1u << lane) - 1u;
-    unsigned sink = 0u, wu0 = 0u, wu1 = 0u, wu2 = 0u, wu3 = 0u, wu4 = 0u, wu5 = 0u;
-    __syncwarp();
-    for (int i = 0; i < n;) {
-        const int cnt = min(4, n - i);
-        unsigned pk = 0;
-        { const int j = i + slot; if (slot < cnt) pk = (n - j <= LEAN_RING) ? s_ring1[j & (LEAN_RING - 1)] : reg[j]; }
-        const int xx = (int)(pk & 0xffff) + ox, yy = (int)(pk >> 16) + oy, q = yy * w + xx;
-        const bool valid = slot < cnt && (unsigned)xx < (unsigned)w && (unsigned)yy < (unsigned)h;
-        uint4 v = make_uint4(__float_as_uint(NOTDEF_F), 0u, 0u, 1u);
-        if (valid) v = *reinterpret_cast<const uint4*>(pix + q);
-        const unsigned peers = __match_any_sync(0xffffffffu, valid ? q : ~lane);     // under the load
-        sink ^= wu0 ^ wu1 ^ wu2 ^ wu3 ^ wu4 ^ wu5;                                   // last step's warm-up loads have landed by now
-        if (dirty) { th = fast_atan2_deg(sumdy, sumdx); rM = rsqrtf(sumdx * sumdx + sumdy * sumdy); dirty = false; }
-        const float a = __uint_as_float(v.x), cx = __uint_as_float(v.y), cy = __uint_as_float(v.z);
-        unsigned pending = __ballot_sync(0xffffffffu, valid && a != NOTDEF_F && v.w == 0u);
-        while (pending) {
-            const bool mep = (pending >> lane) & 1u;
-            const float d = fabsf(th - a);
-            const float e = d > 270.f ? 360.f - d : d;
-            bool pass = e <= pdeg;
-            const bool near = fabsf(e - pdeg) < 2e-3f || fabsf(d - 270.f) < 2e-3f;
-            if (__any_sync(0xffffffffu, mep && near)) { if (near) pass = l_aligned_rad((double)a * L_DEG, (double)th * L_DEG, prec); }
-            const unsigned P = __ballot_sync(0xffffffffu, mep && pass);
-            if (!P) break;                                        // nobody passes at the current angle: all rejected
-            const int k0 = __ffs(P) - 1;
-            const unsigned P1 = P & ~__ballot_sync(0xffffffffu, pass && mep && (peers & P & lt) != 0u);   // first holders among the passing lanes
-            const float x = (float)__popc(P1 & lt) * rM;          // (vectors the scan can have added before this lane) / |S|
-            bool robust = false;
-            if (rob_ok && x <= 0.5f) { const float B = coef * x + 0.0215f; robust = pass ? (e <= pdeg - B) : (e >= pdeg + B); }
-            const unsigned NR = __ballot_sync(0xffffffffu, mep && lane > k0 && !robust);
-            const unsigned below = NR ? ((NR & (0u - NR)) - 1u) : 0xffffffffu;       // lanes before the first non-robust one
-            const unsigned A = P1 & below;                        // accepted in this round, in scan order
-            for (unsigned Tm = A; Tm; Tm &= Tm - 1u) {            // the sums, in scan order
-                const int mm = __ffs(Tm) - 1;
-                sumdx += __shfl_sync(0xffffffffu, cx, mm); sumdy += __shfl_sync(0xffffffffu, cy, mm);
-            }
-            if ((A >> lane) & 1u) {
-                const int pos = n + __popc(A & lt);
-                const unsigned me = (unsigned)xx | ((unsigned)yy << 16);
-                s_ring1[pos & (LEAN_RING - 1)] = me; reg[pos] = me; pix[q].used = 1u;
-                const int xa = max(xx - 1, 0), xb = min(xx + 1, w - 1), ya = max(yy - 1, 0), yb = min(yy + 1, h - 1);
-                const unsigned* r0 = reinterpret_cast<const unsigned*>(pix + ya * w), * r1 = reinterpret_cast<const unsigned*>(pix + yy * w), * r2 = reinterpret_cast<const unsigned*>(pix + yb * w);
-                asm volatile("ld.global.ca.u32 %0, [%1];" : "=r"(wu0) : "l"(r0 + 4 * xa));
-                asm volatile("ld.global.ca.u32 %0, [%1];" : "=r"(wu1) : "l"(r0 + 4 * xb));
-                asm volatile("ld.global.ca.u32 %0, [%1];" : "=r"(wu2) : "l"(r1 + 4 * xa));
-                asm volatile("ld.global.ca.u32 %0, [%1];" : "=r"(wu3) : "l"(r1 + 4 * xb));
-                asm volatile("ld.global.ca.u32 %0, [%1];" : "=r"(wu4) : "l"(r2 + 4 * xa));
-                asm volatile("ld.global.ca.u32 %0, [%1];" : "=r"(wu5) : "l"(r2 + 4 * xb));
-            }
-            n += __popc(A);
-            pending &= ~below;                                    // everything before the first non-robust lane is resolved
-            pending &= ~__ballot_sync(0xffffffffu, mep && (peers & A) != 0u);        // later holders of accepted pixels
-            dirty = true;
-            if (pending) { th = fast_atan2_deg(sumdy, sumdx); rM = rsqrtf(sumdx * sumdx + sumdy * sumdy); dirty = false; }
-        }
-        __syncwarp();
-        i += cnt;
-    }
-    if (dirty) th = fast_atan2_deg(sumdy, sumdx);
-    if (sink == 0x9e3779b9u && n < 0) reg[0] = sink;             // keeps the warm-up loads alive (never true)
-    *reg_angle_out = (double)th * L_DEG;
-    return n;
-}
-
 __device__ __forceinline__ double l_angle_diff_signed(double a, double b) {
     double d = a - b;
     while (d <= -L_PI) d += L_2PI;
@@ -788,7 +670,7 @@ __device__ __forceinline__ double l_distsq(double x1, double y1, double x2, doub
 template <int SOLO> __device__ __noinline__ bool l_reduce_region_radius(int* n_io, double reg_angle, double prec, double p, LRect* rec, double density, double density_th) {
     const int lane = threadIdx.x & 31, w = s_W.w;
     int n = *n_io;
-    if ((SOLO == 0 || SOLO == 3 || SOLO == 4) && s_W.mode == 0) {  // speculative attempt: keep the list as it is (the commit validates every pixel ever accepted) and work on a copy
+    if (SOLO == 0 && s_W.mode == 0) {  // speculative attempt: keep the list as it is (the commit validates every pixel ever accepted) and work on a copy
         if (2 * n + s_W.nasm > s_W.cap) { s_W.abort = 1; return false; }
         for (int i = lane; i < n; i += 32) s_W.reg[n + i] = s_W.reg[i];
         s_W.reg += n; s_W.cap -= n;
@@ -865,7 +747,6 @@ template <int SOLO> __device__ __noinline__ bool l_refine(int* n_io, double* reg
     int n = *n_io;
     double density = (double)n / (l_dist(rec->x1, rec->y1, rec->x2, rec->y2) * rec->width);
     if (density >= density_th) return true;
-    if constexpr (SOLO == 3) { if (lane == 0) s_W.dirty = 1; }      // pixels get released: attempts that assumed them used cannot be validated
     const unsigned* reg = s_W.reg; const float* __restrict__ ang = s_W.ang;
     const unsigned p0 = reg[0];
     const int sx = p0 & 0xffff, sy = p0 >> 16;
@@ -897,12 +778,10 @@ template <int SOLO> __device__ __noinline__ bool l_refine(int* n_io, double* reg
     const double mean_angle = sum / (double)cnt;
     const double tau = 2.0 * sqrt((s_sum - 2.0 * mean_angle * sum) / (double)cnt + mean_angle * mean_angle);
     __syncwarp();
-    if ((SOLO == 0 || SOLO == 3) && s_W.mode == 0) { s_W.reg += n; s_W.cap -= n; }   // speculative: the first list stays (validated at commit), the regrown one follows it
-    if constexpr (SOLO == 2) n = l_region_grow_lean(sx, sy, tau, reg_angle_io);
-    else if constexpr (SOLO == 3) n = l_region_grow_v3(sx, sy, tau, reg_angle_io);
-    else n = l_region_grow<SOLO>(sx, sy, tau, reg_angle_io);
+    if (SOLO == 0 && s_W.mode == 0) { s_W.reg += n; s_W.cap -= n; }   // speculative: the first list stays (validated at commit), the regrown one follows it
+    n = l_region_grow<SOLO>(sx, sy, tau, reg_angle_io);
     if (n < 0) { *n_io = 0; return false; }
-    if ((SOLO == 0 || SOLO == 3) && s_W.mode == 0) s_W.acc += n;
+    if (SOLO == 0 && s_W.mode == 0) s_W.acc += n;
     *n_io = n;
     if (n < 2) return false;
     l_region2rect<SOLO>(n, *reg_angle_io, prec, p, rec);
@@ -1442,1060 +1321,6 @@ __global__ void __launch_bounds__(32, SSLPL_SOLO_MINB) k_lsd_regions_solo(const 
   }
 }
 
-// The same loop over the frame's seeds with the LEAN region growing (l_region_grow_lean).  Alone it takes the same time as
-// k_lsd_regions_solo (49.5 vs 50.6 ms for 148 frames), with several launches overlapping it is slower (38.5 vs 29.2 ms per bench
-// step): it executes 5 % MORE warp instructions (the lazy-angle bookkeeping costs what the removed FP64 saved), and a lone warp's time
-// is instructions x ~8 cycles.  Kept for A/B runs (SSLPL_WALKER_LEAN=1) and as the base of the v3 and lane-parallel growth.
-__global__ void __launch_bounds__(32, 28) k_lsd_regions_lean(const __grid_constant__ LineGeom g, LineWs ws, int nframes) {
-    const int lane = threadIdx.x;
-  for (;;) {
-    int f = 0;
-    if (lane == 0) f = atomicAdd(ws.rejctl + 2, 1);
-    f = __shfl_sync(0xffffffffu, f, 0);
-    if (f >= nframes) break;
-    __syncwarp();
-    WalkCtx& W = s_W1;
-    if (lane == 0) {
-        W.w = g.sw; W.h = g.sh; W.mode = 2; W.abort = 0; W.nasm = 0; W.acc = 0; W.cap = (int)g.pix_stride; W.ticket = 1u; W.seq = 0;
-        W.ang = ws.angdeg + f * g.pix_stride; W.mod = ws.modgrad + f * g.pix_stride;
-        W.pix = ws.pix + f * g.pix_stride; W.reg = ws.reg + f * g.pix_stride; W.base0 = W.reg; W.cs0 = ws.cs0 + f * g.pix_stride; W.bits = nullptr;
-    }
-    __syncwarp();
-    const LPix* pix = ws.pix + f * g.pix_stride;
-    const unsigned* seeds = ws.seeds + f * g.pix_stride;
-    const int ns = ws.nseeds[f];
-    double* jobs = ws.jobs + (long long)f * g.seg_cap * 13;
-    int nj = 0;
-    for (int sb = 0; sb < ns; sb += 32) {
-        const bool have = sb + lane < ns;
-        const unsigned mine = have ? seeds[sb + lane] : 0u;                   // 32 seeds per coalesced load
-        unsigned umask = __ballot_sync(0xffffffffu, !have || pix[mine].used != 0u); // their `used` state, one round trip
-        while (~umask) {                                    // angle != NOTDEF holds for every seed
-            const int j = __ffs(~umask) - 1;
-            umask |= (2u << j) - 1u;                        // seeds up to j are done
-            const unsigned idx = __shfl_sync(0xffffffffu, mine, j);
-            double reg_angle;
-            int n = l_region_grow_lean((int)(idx % (unsigned)g.sw), (int)(idx / (unsigned)g.sw), g.prec, &reg_angle);
-#ifdef SSLPL_V3_DEBUG
-            if ((int)idx == g.dbg_seed) { __syncwarp(); for (int i = lane; i < n; i += 32) printf("L1 %d %u %u\n", i, W.reg[i] & 0xffff, W.reg[i] >> 16); __syncwarp(); }
-#endif
-            umask |= __ballot_sync(0xffffffffu, !have || pix[mine].used != 0u);    // the region may have swallowed later seeds
-            if (n < g.min_reg_size) continue;
-            LRect rec;
-            l_region2rect<2>(n, reg_angle, g.prec, g.p, &rec);
-            const int n0 = n;
-            const bool okr = l_refine<2>(&n, &reg_angle, g.prec, g.p, &rec, 0.7);
-            umask = ((2u << j) - 1u) | __ballot_sync(0xffffffffu, !have || pix[mine].used != 0u);   // refine can release and re-take pixels
-            if (!okr) continue;
-            if (nj < g.seg_cap) l_emit_job(g, jobs + (long long)nj * 13, rec, idx, n0, lane);
-            nj++;
-        }
-    }
-    if (lane == 0) { ws.njobs[f] = min(nj, g.seg_cap); if (nj > g.seg_cap) atomicOr(ws.err, DERR_LSD_OVERFLOW); }
-    __syncwarp();
-  }
-}
-
-
-// =================================================================================================
-// Multi-warp region walker, v3 (round 2b).  Same idea as k_lsd_regions — regions are grown AHEAD of the sequential order
-// by several warps and retired strictly IN that order — with the two costs that dominated it removed (measured on one
-// 640x480 frame: 58 % of the frame's cycles under the commit lock, 3600 cycles per commit, every invalid attempt regrown
-// under that lock while 15 warps wait):
-//   * RETIRING AN ATTEMPT IS O(1).  "Used" is not a bitmap that a commit has to fill but a property of the ticket found in
-//     LPix.used: a ticket (rank, try) of a retired rank is USED iff that try is the one the rank committed with.  That
-//     is try 0 unless the rank's bit is set in a 64k-bit exception map in shared memory (then one byte per rank in global
-//     memory says which try, if any).  So a commit writes one byte, maybe one bit, advances `turn`; there are no lists to
-//     validate, no bits to set, no list storage per slot (the lists belong to the worker and die with the attempt);
-//   * validity is tracked where it is decided: an attempt that takes a pixel from a live attempt of higher rank POISONS it;
-//     an attempt that meets a pixel held by a live attempt of LOWER rank assumes it used and records that attempt as a
-//     dependency (two at most), valid iff it commits with that very try without ever having released a pixel;
-//   * warp 0 is the CONTROL warp (claims seeds in order into a ring of 256 tiny slots (more ranks in flight only add wasted speculation: 14.4-15.0 ms per frame at 128-256, 17.9 at 1024, 30.7 at 4096), retires the head); the others are
-//     workers that pick the lowest runnable slot.  No locks.  An invalid attempt goes back to the ring with try + 1; the
-//     head of the ring can neither meet a live lower rank nor be poisoned, so its attempt always commits.
-// Region growing is the lean form (float-degree test, lazy angle, list tail in shared memory) with tickets taken by CAS whose
-// result is looked at one step later.
-// =================================================================================================
-constexpr int V3_MAXW = 16;            // warps per CTA: 1 control + up to 15 workers
-#ifndef SSLPL_V3_RING
-#define SSLPL_V3_RING 256
-#endif
-constexpr int V3_RING = SSLPL_V3_RING; // ranks in flight (claimed, not retired)
-constexpr int V3_LIST = 8192;          // list entries of a worker (ws.sreg); bigger regions are regrown as head with the frame-sized list
-constexpr int V3_LRING = 512;          // tail of the worker's list kept in shared memory
-constexpr int V3_RANKS = 65536;        // ranks per frame (exception bits, rcode bytes)
-constexpr int V3_DPOOL = 131072;       // per frame: list entries of the attempts that released pixels, kept until they retire
-static_assert(V3_MAXW * V3_LIST <= WALK_RING * WALK_SLOT_CAP, "the workers' lists live in ws.sreg");
-enum { V3_EMPTY = 0, V3_READY = 1, V3_RUNNING = 2, V3_DONE = 3, V3_PRESUMED = 4, V3_VOID = 5 };
-enum { V3F_JOB = 1, V3F_DIRTY = 2, V3F_RAN = 4 };      // slot flags; bits 4..5 = number of dependencies
-
-struct V3Shared {
-    volatile unsigned turn, nclaims;     // ranks [turn, nclaims) are live; slot of rank r = r % V3_RING
-    unsigned cursor;
-    int ns, nj, all_claimed, frame, done, nready, scanhint, win_base, overflow;
-    unsigned win[WALK_WIN];
-    int state[V3_RING];
-    int seed[V3_RING];
-    int wait[V3_RING];                   // READY: runnable once turn > wait
-    int dl_off[V3_RING], dl_n[V3_RING];  // DONE, dirty: where the pixels it ever accepted are kept until it retires (ws.dlist)
-    int dl_used;
-    int nblocked;                        // READY slots that wait for an attempt of lower rank (they do not count against the claim throttle)
-    unsigned dep[V3_RING][2];
-    unsigned char tryno[V3_RING], poison[V3_RING], flag[V3_RING];
-    unsigned excbits[V3_RANKS / 32];     // rank retired with something else than "try 0 committed" although a try ran
-    unsigned lring[1];                   // [warps][V3_LRING] follows
-};
-extern __shared__ __align__(16) unsigned char s_v3raw[];
-__device__ __forceinline__ V3Shared& v3s() { return *reinterpret_cast<V3Shared*>(s_v3raw); }
-
-__device__ __forceinline__ int v3_rank(unsigned m) { return (int)(m & 0xffffffu) - 1; }
-__device__ __forceinline__ int v3_try(unsigned m) { return (int)((m >> 24) & 0x7fu); }
-// What is a foreign, non-zero ticket to the attempt of rank `myseq`?  0 free (stale), 1 used (committed), 2 held by a live attempt
-// of lower rank, 3 held by a live attempt of higher rank.
-__device__ __forceinline__ int v3_classify(unsigned m, int myseq, const unsigned char* __restrict__ rcode) {
-    V3Shared& S = v3s();
-    if (m & 0x80000000u) return 0;                                // released by its attempt
-    const int r = v3_rank(m), y = v3_try(m);
-    if (r >= (int)S.turn) {
-        const int yy = *reinterpret_cast<volatile unsigned char*>(&S.tryno[r & (V3_RING - 1)]);
-        if (r >= (int)S.turn) {                                   // still live: the slot was rank r's when it was read
-            if (yy != y) return 0;                                // an earlier, abandoned try of a live rank
-            return r < myseq ? 2 : 3;
-        }
-    }
-    if (!((reinterpret_cast<volatile unsigned*>(S.excbits)[r >> 5] >> (r & 31)) & 1u)) return y == 0 ? 1 : 0;
-    const unsigned code = __ldcg(rcode + r);
-    return (code != 0xffu && (int)(code & 0x7fu) == y) ? 1 : 0;
-}
-__device__ __forceinline__ void v3_poison(unsigned m) {
-    V3Shared& S = v3s();
-    const int r = v3_rank(m);
-    if (r >= (int)S.turn) *reinterpret_cast<volatile unsigned char*>(&S.poison[r & (V3_RING - 1)]) = (unsigned char)(v3_try(m) + 1);
-}
-// Result of the atomic issued one step earlier: -1 the pixel is mine, >= 0 the live attempt of lower rank that holds it (repeat after
-// it has retired), -2 lost to anybody else (repeat at once).
-__device__ __forceinline__ int v3_take_resolve(const WalkCtx& W, LTake& t, const unsigned char* rcode) {
-    if (!t.pend) return -1;
-    t.pend = false;
-    const unsigned old = t.old;
-#ifdef SSLPL_V3_DEBUG
-    if ((W.dbg & 16) && t.q == W.nasm) printf("RES T %x seen %x old %x mode %d turn %u\n", W.ticket, t.seen, old, W.mode, v3s().turn);
-#endif
-    if (W.mode != 0 || old == t.seen) {
-        // mine now.  Whoever held it alive, or had held and released it, with a higher rank grew over a pixel that is mine: poisoned
-        const unsigned o = old & 0x7fffffffu;
-        if (o != 0u && o != W.ticket && v3_classify(o, W.seq, rcode) == 3) v3_poison(o);
-        return -1;
-    }
-    if (old != 0u && v3_classify(old, W.seq, rcode) == 2) return v3_rank(old);
-    return -2;
-}
-
-__device__ __noinline__ int l_region_grow_v3(int sx, int sy, double prec, double* reg_angle_out) {
-    WalkCtx& W = s_Wc[threadIdx.x >> 5];
-    V3Shared& S = v3s();
-    unsigned* ring = S.lring + (threadIdx.x >> 5) * V3_LRING;
-    const int lane = threadIdx.x & 31, w = W.w, h = W.h;
-    LPix* pix = W.pix; unsigned* reg = W.reg;
-    const unsigned char* rcode = reinterpret_cast<const unsigned char*>(W.bits);      // per-rank commit codes of this frame (global)
-    const unsigned T = W.ticket; const int myseq = W.seq; const bool spec = W.mode == 0;
-    const int cap = W.cap;
-    const int sq = sy * w + sx;
-    LTake tk; tk.pend = false; tk.q = 0; tk.seen = 0u; tk.old = 0u;
-    int failrank = -1;
-    {
-        int fail = 0;
-        if (lane == 0) {
-            const unsigned pk0 = (unsigned)sx | ((unsigned)sy << 16);
-            reg[0] = pk0; ring[0] = pk0;
-            const unsigned m0 = __ldcg(&pix[sq].used);
-            if (m0 != T) {
-                const int c = m0 == 0u ? 0 : v3_classify(m0, myseq, rcode);
-                if (c == 1) fail = 4;                                          // committed meanwhile: nothing to grow
-                else if (c == 2) { fail = 3; W.conflict = (int)m0; }           // under a live attempt of lower rank: presumed swallowed
-                else {
-                    l_take_issue(W, tk, sq, m0);
-                    const int r = v3_take_resolve(W, tk, rcode);
-                    if (r != -1) { fail = 2; W.conflict = r >= 0 ? r : -1; }
-                }
-            }
-        }
-        fail = __shfl_sync(0xffffffffu, fail, 0);
-        if (fail) { if (lane == 0) W.abort = fail; __syncwarp(); return -1; }
-    }
-    float th = __ldg(W.ang + sq);
-    const float2 c0 = __ldg(W.cs0 + sq);
-    float sumdx = c0.x, sumdy = c0.y;
-    float rM = rsqrtf(sumdx * sumdx + sumdy * sumdy);
-    bool dirty = false;
-    int n = 1;
-    const float pdeg = (float)(prec * (180.0 / L_PI));
-    const float coef = (float)(57.2958 * 1.0002 * sin(prec + 0.0006));
-    const bool rob_ok = prec < 0.78;
-    const int slot = lane >> 3, nb = (lane & 7) + ((lane & 7) >= 4 ? 1 : 0);
-    const int ox = nb % 3 - 1, oy = nb / 3 - 1;
-    const unsigned lt = (1u << lane) - 1u;
-    __syncwarp();
-    for (int i = 0; i < n;) {
-        const int cnt = min(4, n - i);
-        unsigned pk = 0;
-        { const int j = i + slot; if (slot < cnt) pk = (n - j <= V3_LRING) ? ring[j & (V3_LRING - 1)] : reg[j]; }
-        const int xx = (int)(pk & 0xffff) + ox, yy = (int)(pk >> 16) + oy, q = yy * w + xx;
-        const bool valid = slot < cnt && (unsigned)xx < (unsigned)w && (unsigned)yy < (unsigned)h;
-        uint4 v = make_uint4(__float_as_uint(NOTDEF_F), 0u, 0u, 0u);
-        if (valid) v = __ldcg(reinterpret_cast<const uint4*>(pix + q));          // record + ticket (tickets change under atomics: L2)
-        const unsigned peers = __match_any_sync(0xffffffffu, valid ? q : ~lane);
-        { const int r = v3_take_resolve(W, tk, rcode); if (r != -1) failrank = (r >= 0 && r > failrank) ? r : (failrank >= 0 ? failrank : r); }
-        if (dirty) { th = fast_atan2_deg(sumdy, sumdx); rM = rsqrtf(sumdx * sumdx + sumdy * sumdy); dirty = false; }
-        const float a = __uint_as_float(v.x), cx = __uint_as_float(v.y), cy = __uint_as_float(v.z);
-        const unsigned m = v.w;
-        bool cand = false, lower = false;
-        if (valid && a != NOTDEF_F && m != T) {
-            if (m == 0u) cand = true;
-            else { const int c = v3_classify(m, myseq, rcode); cand = c == 0 || c == 3; lower = c == 2; }
-        }
-#ifdef SSLPL_V3_DEBUG
-        if ((W.dbg & 16) && valid && q == W.nasm) printf("SEE T %x m %x cand %d lower %d turn %u\n", T, m, (int)cand, (int)lower, S.turn);
-#endif
-        for (unsigned lm = __ballot_sync(0xffffffffu, lower); lm;) {              // remember whose pixels were assumed used
-            const unsigned t = __shfl_sync(0xffffffffu, m, __ffs(lm) - 1);
-            if (lane == 0) {
-                const int nd = W.ndeps;
-                if (!((nd > 0 && W.dep[0] == t) || (nd > 1 && W.dep[1] == t))) { if (nd < 2) { W.dep[nd] = t; W.ndeps = nd + 1; } else W.abort = 5; }
-            }
-            lm &= ~__ballot_sync(0xffffffffu, lower && m == t);
-        }
-        unsigned pending = __ballot_sync(0xffffffffu, cand);
-        while (pending) {
-            const bool mep = (pending >> lane) & 1u;
-            const float d = fabsf(th - a);
-            const float e = d > 270.f ? 360.f - d : d;
-            bool pass = e <= pdeg;
-            const bool near = fabsf(e - pdeg) < 2e-3f || fabsf(d - 270.f) < 2e-3f;
-            if (__any_sync(0xffffffffu, mep && near)) { if (near) pass = l_aligned_rad((double)a * L_DEG, (double)th * L_DEG, prec); }
-            const unsigned P = __ballot_sync(0xffffffffu, mep && pass);
-            if (!P) break;
-            const int k0 = __ffs(P) - 1;
-            const unsigned P1 = P & ~__ballot_sync(0xffffffffu, pass && mep && (peers & P & lt) != 0u);
-            const float x = (float)__popc(P1 & lt) * rM;
-            bool robust = false;
-            if (rob_ok && x <= 0.5f) { const float B = coef * x + 0.0215f; robust = pass ? (e <= pdeg - B) : (e >= pdeg + B); }
-            const unsigned NR = __ballot_sync(0xffffffffu, mep && lane > k0 && !robust);
-            const unsigned below = NR ? ((NR & (0u - NR)) - 1u) : 0xffffffffu;
-            const unsigned A = P1 & below;
-            if (n + __popc(A) > cap) { if (lane == 0) W.abort = 1; __syncwarp(); return -1; }
-            for (unsigned Tm = A; Tm; Tm &= Tm - 1u) {
-                const int mm = __ffs(Tm) - 1;
-                sumdx += __shfl_sync(0xffffffffu, cx, mm); sumdy += __shfl_sync(0xffffffffu, cy, mm);
-            }
-            if ((A >> lane) & 1u) {
-                const int pos = n + __popc(A & lt);
-                const unsigned me = (unsigned)xx | ((unsigned)yy << 16);
-                ring[pos & (V3_LRING - 1)] = me; reg[pos] = me;
-#ifdef SSLPL_V3_DEBUG
-                if ((W.dbg & 16) && q == W.nasm) printf("TAKE T %x q (%d,%d) seen %x mode %d pos %d turn %u\n", T, xx, yy, m, W.mode, pos, S.turn);
-#endif
-                l_take_issue(W, tk, q, m);
-            }
-            n += __popc(A);
-            pending &= ~below;
-            pending &= ~__ballot_sync(0xffffffffu, mep && (peers & A) != 0u);
-            dirty = true;
-            if (pending) { th = fast_atan2_deg(sumdy, sumdx); rM = rsqrtf(sumdx * sumdx + sumdy * sumdy); dirty = false; }
-        }
-        __syncwarp();
-        if (spec && (__any_sync(0xffffffffu, failrank != -1) || W.abort)) break;    // lost a pixel / too many dependencies: stop now
-        if (spec && !(W.dbg & 64) && *reinterpret_cast<volatile unsigned char*>(&S.poison[myseq & (V3_RING - 1)]) == (unsigned char)((T >> 24) + 1u)) { if (lane == 0) { W.abort = 2; W.conflict = -1; } __syncwarp(); return -1; }   // a lower rank took one of my pixels: this try is void
-        i += cnt;
-    }
-    { const int r = v3_take_resolve(W, tk, rcode); if (r != -1) failrank = (r >= 0 && r > failrank) ? r : (failrank >= 0 ? failrank : r); }
-    const bool lostany = __any_sync(0xffffffffu, failrank != -1);
-    failrank = __reduce_max_sync(0xffffffffu, failrank);
-    if (W.abort) return -1;
-    if (lostany) { if (lane == 0) { W.abort = 2; W.conflict = failrank >= 0 ? failrank : -1; } __syncwarp(); return -1; }
-    if (dirty) th = fast_atan2_deg(sumdy, sumdx);
-    *reg_angle_out = (double)th * L_DEG;
-    return n;
-}
-
-// grow + fit + refine one seed as attempt (W.seq, try): 1 = candidate rectangle in *rec, 0 = no job, -1 = abandoned (W.abort)
-__device__ __noinline__ int v3_one_region(const LineGeom& g, unsigned idx, LRect* rec, int* n0) {
-    WalkCtx& W = s_Wc[threadIdx.x >> 5];
-    double reg_angle;
-    int n = l_region_grow_v3((int)(idx % (unsigned)g.sw), (int)(idx / (unsigned)g.sw), g.prec, &reg_angle);
-    if (n < 0) return -1;
-    *n0 = n;
-    W.acc = n;
-#ifdef SSLPL_V3_DEBUG
-    if ((int)idx == g.dbg_seed) { __syncwarp(); for (int i = (threadIdx.x & 31); i < n; i += 32) printf("L3 %d %u %u %u\n", i, W.reg[i] & 0xffff, W.reg[i] >> 16, W.ticket); __syncwarp(); }
-#endif
-    if (n < g.min_reg_size) return 0;
-    l_region2rect<3>(n, reg_angle, g.prec, g.p, rec);
-    const bool okr = l_refine<3>(&n, &reg_angle, g.prec, g.p, rec, 0.7);
-    if (W.abort) return -1;
-    return okr ? 1 : 0;
-}
-
-// One pass of the RETIRER over the head of the ring (a whole warp; returns whether anything moved).  Runs of PRESUMED slots — the
-// seeds a region swallowed while it was live come right behind it in seed order — are looked at 32 at a time (one ticket load per
-// lane) and retired together; DONE / VOID slots one by one (their validity can depend on the slot before).
-__device__ bool v3_retire_pass(const LineGeom& g, const LineWs& ws, int f, unsigned char* rcode, unsigned long long* cnt) {
-    V3Shared& S = v3s();
-    const int lane = threadIdx.x & 31;
-    const LPix* pix = ws.pix + (long long)f * g.pix_stride;
-    bool progress = false;
-    for (;;) {
-        const unsigned t = S.turn, nc = S.nclaims;
-        if (t >= nc) break;
-        const int k = (int)(t & (V3_RING - 1));
-        const int st = *reinterpret_cast<volatile int*>(&S.state[k]);
-        if (st == V3_PRESUMED) {
-            const unsigned r = t + (unsigned)lane;
-            const int kk = (int)(r & (V3_RING - 1));
-            const bool pres = r < nc && *reinterpret_cast<volatile int*>(&S.state[kk]) == V3_PRESUMED;
-            const unsigned pm = __ballot_sync(0xffffffffu, pres);
-            const int len = __ffs(~pm) - 1 < 0 ? 32 : __ffs(~pm) - 1;            // leading PRESUMED slots
-            __threadfence_block();
-            int c = 0;
-            if (lane < len) { const unsigned m = __ldcg(&pix[S.seed[kk]].used); c = m == 0u ? 0 : v3_classify(m, (int)r, rcode); }
-            const unsigned sw = __ballot_sync(0xffffffffu, lane < len && c == 1);
-            const int nsw = __ffs(~sw) - 1 < 0 ? 32 : __ffs(~sw) - 1;             // leading swallowed ones: they retire together
-            bool ran = false;
-            if (lane < nsw) {
-                rcode[r] = 0xffu;
-                ran = (S.flag[kk] & V3F_RAN) != 0;
-                if (ran) atomicOr(&S.excbits[r >> 5], 1u << (r & 31));
-                *reinterpret_cast<volatile int*>(&S.state[kk]) = V3_EMPTY;
-            }
-            if (__any_sync(0xffffffffu, ran)) __threadfence(); else __threadfence_block();
-            __syncwarp();
-            if (nsw > 0) { if (lane == 0) S.turn = t + (unsigned)nsw; cnt[4] += (unsigned long long)nsw; progress = true; }
-            if (nsw < len) {                                                       // the new head was not swallowed after all: it grows now
-                if (lane == nsw) { S.wait[kk] = -1; atomicMin(&S.scanhint, (int)r); __threadfence_block(); atomicAdd(&S.nready, 1); *reinterpret_cast<volatile int*>(&S.state[kk]) = V3_READY; }
-                cnt[5]++; progress = true;
-                __syncwarp();
-                break;
-            }
-            __syncwarp();
-            continue;
-        }
-        if (st != V3_DONE && st != V3_VOID) break;
-        __threadfence_block();
-        bool relbad = false;                                      // a pixel it accepted and released is used by a region of lower rank
-        if (st == V3_DONE && (S.flag[k] & V3F_DIRTY) && S.dl_n[k] > 0) {
-            const unsigned* dl = ws.dlist + (long long)f * V3_DPOOL + S.dl_off[k];
-            const int nn = S.dl_n[k];
-            bool bad = false;
-            for (int i = lane; i < nn; i += 32) {
-                const unsigned pk = __ldcg(dl + i);
-                const unsigned tg = __ldcg(&pix[(int)(pk >> 16) * g.sw + (int)(pk & 0xffff)].used);
-                if (tg != 0u && !(tg & 0x80000000u) && v3_rank(tg) != (int)t && v3_classify(tg, (int)t, rcode) == 1) bad = true;
-            }
-            relbad = __any_sync(0xffffffffu, bad);
-        }
-        int act = 0;                                              // 1 retire (| 4 with a job, | 8 exception), 2 back to READY
-        if (lane == 0) {
-            const int y = S.tryno[k], fl = S.flag[k];
-            if (st == V3_DONE) {
-                const bool pois = *reinterpret_cast<volatile unsigned char*>(&S.poison[k]) == (unsigned char)(y + 1);
-                bool ok = !pois && !relbad;
-                const int nd = (fl >> 4) & 3;
-                for (int d = 0; d < nd && ok; d++) { const unsigned tk = S.dep[k][d]; ok = __ldcg(rcode + v3_rank(tk)) == (unsigned)v3_try(tk); }   // committed with that try, nothing released
-#ifdef SSLPL_V3_DEBUG
-                if ((g.dbg & 16) && t < 64) printf("RET rank %u try %d flags %x poison %d -> %s\n", t, y, fl, (int)S.poison[k], ok ? "commit" : "redo");
-#endif
-                if (ok) {
-                    rcode[t] = (unsigned char)(y | ((fl & V3F_DIRTY) ? 0x80 : 0));
-                    if (y != 0) S.excbits[t >> 5] |= 1u << (t & 31);
-                    act = 1 | ((fl & V3F_JOB) ? 4 : 0) | (y != 0 ? 8 : 0);
-                    cnt[0]++;
-                } else {
-                    S.tryno[k] = (unsigned char)min(y + 1, 126); S.poison[k] = 0; S.flag[k] = V3F_RAN; S.wait[k] = -1;
-                    act = 2;
-                    cnt[pois ? 1 : 2]++;
-                }
-            } else {
-                rcode[t] = 0xffu;
-                if (fl & V3F_RAN) S.excbits[t >> 5] |= 1u << (t & 31);
-                act = 1 | ((fl & V3F_RAN) ? 8 : 0);
-                cnt[3]++;
-            }
-        }
-        act = __shfl_sync(0xffffffffu, act, 0);
-        if (act & 1) {
-            if (act & 4) {
-                const int nj = S.nj;
-                if (nj < g.seg_cap && lane < 13) ws.jobs[((long long)f * g.seg_cap + nj) * 13 + lane] = __ldcg(ws.sjob + ((long long)f * V3_RING + k) * 13 + lane);
-                if (lane == 0) S.nj = nj + 1;
-            }
-            __syncwarp();
-            if (lane == 0) { if (act & 8) __threadfence(); *reinterpret_cast<volatile int*>(&S.state[k]) = V3_EMPTY; __threadfence_block(); S.turn = t + 1; }
-        } else {
-            if (lane == 0) { atomicMin(&S.scanhint, (int)t); __threadfence_block(); atomicAdd(&S.nready, 1); *reinterpret_cast<volatile int*>(&S.state[k]) = V3_READY; }
-        }
-        __syncwarp();
-        progress = true;
-        if (!(act & 1)) break;                                    // the head runs again: nothing behind it can retire
-    }
-    return progress;
-}
-
-// One pass of the CLAIMER: the next 32 seeds of the ordered list are looked at together (one ticket load per lane) and every one
-// that is not used by a committed region gets the next rank and a slot — READY, or PRESUMED swallowed if it is under a live ticket.
-__device__ bool v3_claim_pass(const LineGeom& g, const LineWs& ws, int f, unsigned char* rcode, int limit = 0) {
-    V3Shared& S = v3s();
-    const int lane = threadIdx.x & 31;
-    const LPix* pix = ws.pix + (long long)f * g.pix_stride;
-    const unsigned* seeds = ws.seeds + (long long)f * g.pix_stride;
-    const int ns = S.ns;
-    if (S.all_claimed) return false;
-    const unsigned nc = S.nclaims;
-    if (nc - S.turn >= (unsigned)(V3_RING - 33)) { if ((g.dbg & 32) && (threadIdx.x & 31) == 0) atomicAdd(ws.wstat + 6, 1ull); return false; }
-    if (*reinterpret_cast<volatile int*>(&S.nready) - *reinterpret_cast<volatile int*>(&S.nblocked) >= (limit ? limit : (((g.dbg >> 8) & 0xff) ? ((g.dbg >> 8) & 0xff) : 1) * (int)(blockDim.x >> 5))) return false;
-    if (nc >= (unsigned)(V3_RANKS - 33)) { if (lane == 0) { S.overflow = 1; S.all_claimed = 1; } __syncwarp(); return true; }
-    const int cur = (int)S.cursor;
-    if (cur >= ns) { if (lane == 0) S.all_claimed = 1; __syncwarp(); return true; }
-    const int i = cur + lane;
-    const bool have = i < ns;
-    const unsigned mine = have ? seeds[i] : 0u;
-    unsigned m = 0; int cls = 1;
-    if (have) { m = __ldcg(&pix[mine].used); cls = m == 0u ? 0 : v3_classify(m, 0x7fffffff, rcode); }     // any live ticket is of lower rank than a new claim
-    const unsigned fm = __ballot_sync(0xffffffffu, have && cls != 1);
-    const int nfree = __popc(__ballot_sync(0xffffffffu, have && cls == 0));
-    if (have && cls != 1) {
-        const unsigned r = nc + (unsigned)__popc(fm & ((1u << lane) - 1u));
-        const int k = (int)(r & (V3_RING - 1));
-        S.seed[k] = (int)mine; S.tryno[k] = 0; S.poison[k] = 0; S.flag[k] = 0; S.wait[k] = -1;
-        if (cls != 0) S.dep[k][0] = m;
-        __threadfence_block();
-        *reinterpret_cast<volatile int*>(&S.state[k]) = cls != 0 ? V3_PRESUMED : V3_READY;
-    }
-    __threadfence_block();
-    __syncwarp();
-    if (lane == 0) {
-        if (nfree) atomicAdd(&S.nready, nfree);
-        S.cursor = (unsigned)min(cur + 32, ns);
-        __threadfence_block();
-        S.nclaims = nc + (unsigned)__popc(fm);
-    }
-    __syncwarp();
-    return true;
-}
-
-__device__ void v3_worker(const LineGeom& g, const LineWs& ws, int f, unsigned char* rcode) {
-    V3Shared& S = v3s();
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    WalkCtx& W = s_Wc[wid];
-    unsigned idle = 0;
-    const bool stat = (g.dbg & 32) != 0;
-    unsigned long long c_busy = 0, c_idle = 0, n_conf = 0, n_cap = 0, n_head = 0, c_abort = 0, c_idle_wait = 0;
-    for (;;) {
-        if (*reinterpret_cast<volatile int*>(&S.done)) break;
-        const long long tw0 = stat ? clock64() : 0;
-        // ---- pick the lowest runnable slot
-        const unsigned t = S.turn, nc = S.nclaims;
-        int from = max((int)t, *reinterpret_cast<volatile int*>(&S.scanhint));
-        int got = -1; bool sawready = false;
-        for (int b = from; b < (int)nc && got < 0; b += 32) {
-            const int r = b + lane;
-            bool ready = false, run = false;
-            if (r < (int)nc) {
-                const int k = r & (V3_RING - 1);
-                ready = *reinterpret_cast<volatile int*>(&S.state[k]) == V3_READY;
-                if (ready) {
-                    // an attempt that lost a pixel to a live attempt of lower rank runs again once that one has finished GROWING (its
-                    // tickets are then what it will commit with, and become a dependency) — not only after it has retired
-                    const int wt = *reinterpret_cast<volatile int*>(&S.wait[k]);
-                    if (wt == r) run = r == (int)t;                            // (out of list space / too many dependencies: only as head)
-                    else {
-                        run = wt < (int)t;
-                        if (!run && !(g.dbg & 128)) { const int sw = *reinterpret_cast<volatile int*>(&S.state[wt & (V3_RING - 1)]); run = sw != V3_READY && sw != V3_RUNNING; }
-                    }
-                }
-            }
-            const unsigned rm = __ballot_sync(0xffffffffu, run);
-            if (!sawready) {
-                const unsigned am = __ballot_sync(0xffffffffu, ready);
-                if (am) sawready = true;
-                else if (lane == 0 && b == from && b + 32 <= (int)nc) atomicCAS(&S.scanhint, from, b + 32);     // nothing READY here: later scans start further on
-            }
-            if (rm) {
-                const int r0 = b + __ffs(rm) - 1;
-                int ok = 0;
-                if (lane == 0) ok = atomicCAS(&S.state[r0 & (V3_RING - 1)], V3_READY, V3_RUNNING) == V3_READY;
-                ok = __shfl_sync(0xffffffffu, ok, 0);
-                if (ok) got = r0; else break;                     // somebody else took it: scan again
-            }
-        }
-        if (got < 0) { idle = min(idle + 1, 8u); __nanosleep(32u << min(idle, 4u)); if (stat) { const long long dd = clock64() - tw0; c_idle += dd; if (sawready) c_idle_wait += dd; } continue; }
-        idle = 0;
-        const long long tw1 = stat ? clock64() : 0;
-        if (stat) c_idle += tw1 - tw0;
-        const int r = got, k = r & (V3_RING - 1);
-        __threadfence_block();
-        const unsigned idx = (unsigned)S.seed[k];
-        const int y = S.tryno[k];
-        const bool head = r == (int)S.turn;                       // nothing of lower rank is live: the frame-sized list is free for it
-        if (lane == 0) {
-            atomicSub(&S.nready, 1);
-            if (S.wait[k] >= 0) atomicSub(&S.nblocked, 1);
-            W.mode = head ? 1 : 0; W.abort = 0; W.conflict = -1; W.seq = r; W.ticket = (unsigned)(r + 1) | ((unsigned)y << 24);
-            W.dirty = 0; W.ndeps = 0; W.nasm = g.dbg_seed; W.acc = 0;
-            if (head) { W.reg = ws.reg + (long long)f * g.pix_stride; W.cap = (int)g.pix_stride; }
-            else { W.reg = ws.sreg + ((long long)f * V3_MAXW + wid) * V3_LIST; W.cap = V3_LIST; }
-            W.base0 = W.reg;
-        }
-        __syncwarp();
-        LRect rec; int n0 = 0;
-        const int res = v3_one_region(g, idx, &rec, &n0);
-        __syncwarp();
-#ifdef SSLPL_V3_DEBUG
-        if ((g.dbg & 16) && lane == 0 && r < 64) printf("W%02d rank %d try %d seed (%d,%d) %s res %d abort %d conflict %d n0 %d ndeps %d [%x %x] dirty %d turn %u\n", wid, r, y, (int)(idx % (unsigned)g.sw), (int)(idx / (unsigned)g.sw), head ? "HEAD" : "spec", res, W.abort, W.conflict, n0, W.ndeps, W.dep[0], W.dep[1], W.dirty, S.turn);
-#endif
-        int res2 = res;
-        if (res >= 0 && W.dirty && W.mode == 0) {
-            // it released pixels: whether one of them belongs to a region of lower rank can only be told when it retires — the pixels
-            // it ever accepted (first growth + re-growth, W.base0[0 .. W.acc)) wait in the frame's pool
-            const int nacc = W.acc;
-            int off = 0;
-            if (lane == 0) off = atomicAdd(&S.dl_used, nacc);
-            off = __shfl_sync(0xffffffffu, off, 0);
-            if (off + nacc > V3_DPOOL) { if (lane == 0) W.abort = 1; res2 = -1; }        // pool exhausted: run it again as head
-            else {
-                unsigned* dst = ws.dlist + (long long)f * V3_DPOOL + off;
-                for (int i = lane; i < nacc; i += 32) dst[i] = W.base0[i];
-                if (lane == 0) { S.dl_off[k] = off; S.dl_n[k] = nacc; }
-            }
-            __syncwarp();
-        } else if (lane == 0) S.dl_n[k] = 0;
-        __syncwarp();
-        if (res2 >= 0) {
-            if (res == 1) l_emit_job(g, ws.sjob + ((long long)f * V3_RING + k) * 13, rec, idx, n0, lane);
-            __syncwarp();
-            if (lane == 0) {
-                const int nd = W.ndeps;
-                for (int d = 0; d < nd; d++) S.dep[k][d] = W.dep[d];
-                S.flag[k] = (unsigned char)(V3F_RAN | (res == 1 ? V3F_JOB : 0) | (W.dirty ? V3F_DIRTY : 0) | (nd << 4));
-                __threadfence();
-                *reinterpret_cast<volatile int*>(&S.state[k]) = V3_DONE;
-            }
-        } else if (lane == 0) {
-            const int ab = W.abort;
-            // (both can also come out of refine's re-growth, after this try has put tickets on pixels: the try number moves on)
-            if (ab == 4) { S.tryno[k] = (unsigned char)min(y + 1, 126); S.flag[k] = V3F_RAN; __threadfence_block(); *reinterpret_cast<volatile int*>(&S.state[k]) = V3_VOID; }   // the seed is used by a committed region
-            else if (ab == 3) { S.tryno[k] = (unsigned char)min(y + 1, 126); S.poison[k] = 0; S.flag[k] = V3F_RAN; S.dep[k][0] = (unsigned)W.conflict; __threadfence_block(); *reinterpret_cast<volatile int*>(&S.state[k]) = V3_PRESUMED; }
-            else {
-                // 2: lost a pixel to a live attempt of lower rank (run again after it has retired) or to a race (run again at once);
-                // 1 / 5: out of list space / more than two dependencies: run again as head
-                S.tryno[k] = (unsigned char)min(y + 1, 126); S.poison[k] = 0; S.flag[k] = V3F_RAN;
-                int wt = ab == 2 ? W.conflict : r;            // wait == r: only as head (turn > r - 1 is checked as wait - 1 < turn below)
-                if (y >= 100) wt = r;
-                S.wait[k] = wt;
-                if (wt >= 0) atomicAdd(&S.nblocked, 1);
-                atomicMin(&S.scanhint, r);
-                __threadfence_block();
-                atomicAdd(&S.nready, 1);
-                *reinterpret_cast<volatile int*>(&S.state[k]) = V3_READY;
-                n_conf++;
-            }
-        }
-        __syncwarp();
-        if (stat) { const long long d = clock64() - tw1; c_busy += d; if (res < 0) c_abort += d; if (head) n_head++; }
-    }
-    if (stat && lane == 0) {
-        atomicAdd(ws.wstat + 6, n_conf); atomicAdd(ws.wstat + 7, n_cap); atomicAdd(ws.wstat + 10, c_busy); atomicAdd(ws.wstat + 11, c_idle);
-        atomicAdd(ws.wstat + 12, c_abort); atomicAdd(ws.wstat + 15, n_head); atomicAdd(ws.wstat + 7, c_idle_wait);
-    }
-}
-
-__global__ void __launch_bounds__(V3_MAXW * 32) k_lsd_regions_v3(const __grid_constant__ LineGeom g, LineWs ws, int nframes) {
-    V3Shared& S = v3s();
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  for (;;) {
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const int f = atomicAdd(ws.rejctl + 2, 1);
-        S.frame = f; S.turn = 0; S.nclaims = 0; S.cursor = 0; S.nj = 0; S.all_claimed = 0; S.done = 0; S.nready = 0; S.nblocked = 0; S.dl_used = 0; S.scanhint = 0; S.win_base = -(1 << 30); S.overflow = 0;
-        S.ns = f < nframes ? ws.nseeds[f] : 0;
-    }
-    for (int i = threadIdx.x; i < V3_RING; i += blockDim.x) { S.state[i] = V3_EMPTY; S.wait[i] = -1; S.tryno[i] = 0; S.poison[i] = 0; S.flag[i] = 0; }
-    for (int i = threadIdx.x; i < V3_RANKS / 32; i += blockDim.x) S.excbits[i] = 0u;
-    __syncthreads();
-    const int f = S.frame;
-    if (f >= nframes) break;
-    unsigned char* rcode = ws.rcode + (long long)f * V3_RANKS;
-    if (lane == 0) {
-        WalkCtx& W = s_Wc[wid];
-        W.w = g.sw; W.h = g.sh; W.dbg = g.dbg;
-        W.ang = ws.angdeg + f * g.pix_stride; W.mod = ws.modgrad + f * g.pix_stride;
-        W.pix = ws.pix + f * g.pix_stride; W.cs0 = ws.cs0 + f * g.pix_stride; W.bits = reinterpret_cast<const unsigned*>(rcode);
-    }
-    __syncwarp();
-    {
-        // warp 0 claims (and works once every seed has been claimed), warp 1 retires, the others work; with two warps, warp 0 does both
-        const bool two = blockDim.x == 64;
-        const bool stat = (g.dbg & 32) != 0;
-        unsigned long long cnt[6] = {0, 0, 0, 0, 0, 0}, c_ret = 0, c_claim = 0, c_idle = 0;
-        if (wid == 0 || (wid == 1 && !two)) {
-            for (;;) {
-                const long long t0 = stat ? clock64() : 0;
-                bool p1 = false, p2 = false;
-                if (wid == 0) p1 = v3_claim_pass(g, ws, f, rcode);
-                const long long t1 = stat ? clock64() : 0;
-                if (wid == 1 || two) {
-                    p2 = v3_retire_pass(g, ws, f, rcode, cnt);
-                    if (S.all_claimed && S.turn >= S.nclaims) { if (lane == 0) { __threadfence_block(); S.done = 1; } __syncwarp(); break; }
-                }
-                if (stat) { const long long t2 = clock64(); if (p1) c_claim += t1 - t0; else c_idle += t1 - t0; if (p2) c_ret += t2 - t1; else c_idle += t2 - t1; }
-                if (wid == 0 && !two && S.all_claimed) break;       // nothing left to claim: become a worker
-                if (!p1 && !p2) __nanosleep(32);
-            }
-            if (stat && lane == 0) {
-                for (int i = 0; i < 6; i++) atomicAdd(ws.wstat + i, cnt[i]);
-                atomicAdd(ws.wstat + 8, c_ret); atomicAdd(ws.wstat + 9, c_claim); atomicAdd(ws.wstat + 14, c_idle);
-                if (wid == 0) atomicAdd(ws.wstat + 13, (unsigned long long)S.nclaims);
-            }
-            if (wid == 0 && !two) v3_worker(g, ws, f, rcode);
-        } else v3_worker(g, ws, f, rcode);
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) { ws.njobs[f] = min(S.nj, g.seg_cap); if (S.nj > g.seg_cap || S.overflow) atomicOr(ws.err, DERR_LSD_OVERFLOW); }
-  }
-}
-
-// =================================================================================================
-// LANE-PARALLEL region walker (round 2b, k_lsd_regions_lanes): ONE WARP PER FRAME, every LANE grows its own region.
-// The one-warp walkers spend ~230 warp instructions per growth step on 32 neighbour tests of ONE region, almost all of it
-// warp-uniform bookkeeping: a lone warp retires one instruction every ~8 cycles, so the stage is bound by instruction count.
-// Here region growing is the plain scalar loop of lsd.cpp run by each lane on a different seed (same protocol as the multi-warp
-// walker v3: ranks in seed order, tickets in LPix.used, poison / dependencies / released-pixel lists, strictly ordered retire —
-// v3_retire_pass and v3_claim_pass are used as they are), so that one warp instruction serves up to 32 regions.  A neighbour is
-// accepted with a SYNCHRONOUS compare-and-swap (nothing to roll back, no "lost a pixel" aborts).  The region angle is lazy per
-// lane (exact fastAtan2 only when a test is within the drift bound of the threshold).  What is cheap per region but long in code
-// — rectangle fit with its ordered double sums, density, refine's release and tau, reduce_region_radius — runs warp-cooperatively
-// with the existing routines (template mode 4) for one finished lane at a time.
-// =================================================================================================
-constexpr int LN_LIST = 4096;          // list entries per lane (32 lanes x 4096 = ws.sreg of a frame); bigger regions run as head on ws.reg
-enum { LN_IDLE = 0, LN_GROW = 1, LN_POST = 2 };
-
-template <int SOLO> __device__ __forceinline__ bool l4_exact_pass(float a, float th, float pdeg, double prec) {
-    const float d = fabsf(th - a);
-    const float e = d > 270.f ? 360.f - d : d;
-    bool pass = e <= pdeg;
-    if (fabsf(e - pdeg) < 2e-3f || fabsf(d - 270.f) < 2e-3f) pass = l_aligned_rad((double)a * L_DEG, (double)th * L_DEG, prec);
-    return pass;
-}
-
-// refine, first half (lsd.cpp refine up to the re-growth): nothing to do if the density is fine (returns true); otherwise every
-// pixel is released, tau is formed from the angles near the seed and, for a speculative attempt, the list pointer moves behind the
-// first list (which stays: every pixel ever accepted is looked at when the attempt retires).
-__device__ __noinline__ bool l4_refine_begin(int n, const LRect* rec, double density_th, double* tau_out) {
-    constexpr int SOLO = 4;
-    const int lane = threadIdx.x & 31, w = s_W.w;
-    const double density = (double)n / (l_dist(rec->x1, rec->y1, rec->x2, rec->y2) * rec->width);
-    if (density >= density_th) return true;
-    if (lane == 0) s_W.dirty = 1;
-    const unsigned* reg = s_W.reg; const float* __restrict__ ang = s_W.ang;
-    const unsigned p0 = reg[0];
-    const int sx = p0 & 0xffff, sy = p0 >> 16;
-    const double xc = (double)sx, yc = (double)sy;
-    const double ang_c = (double)ang[sy * w + sx] * L_DEG;
-    const double width = rec->width;
-    double* s0 = s_st; double* s1 = s_st + 32;
-    const double* sp = s_st + (lane & 1) * 32;
-    double acc = 0; int cnt = 0;
-#pragma unroll 1
-    for (int b = 0; b < n; b += 32) {
-        const int i = b + lane;
-        bool in = false;
-        if (i < n) {
-            const unsigned pk = reg[i]; const int rx = pk & 0xffff, ry = pk >> 16;
-            const float ad = ang[ry * w + rx];
-            l_release<SOLO>(s_W, ry * w + rx);
-            in = l_dist(xc, yc, (double)rx, (double)ry) < width;
-            const double d = l_angle_diff_signed((double)ad * L_DEG, ang_c);
-            s0[lane] = in ? d : 0.0; s1[lane] = in ? d * d : 0.0;
-        }
-        cnt += __popc(__ballot_sync(0xffffffffu, in));
-        __syncwarp();
-        acc = l_chunk_sum<SOLO>(sp, min(32, n - b), acc);
-        __syncwarp();
-    }
-    const double sum = __shfl_sync(0xffffffffu, acc, 0), s_sum = __shfl_sync(0xffffffffu, acc, 1);
-    const double mean_angle = sum / (double)cnt;
-    *tau_out = 2.0 * sqrt((s_sum - 2.0 * mean_angle * sum) / (double)cnt + mean_angle * mean_angle);
-    __syncwarp();
-    return false;
-}
-
-struct LaneAtt {
-    int st, slot, rank, mode, phase, tryno;
-    unsigned T;
-    unsigned* list; int cap;          // the list being grown (behind the first list during a speculative re-growth)
-    int i, n, kacc, n0, acc;
-    float sx, sy, th, rM, pdeg, coefX; double prec; int robok;
-    int ndeps; unsigned dep0, dep1;
-    int abortc, conflict, dirty;
-    unsigned seedidx;
-};
-
-struct LaneFrame { int w, h; LPix* pix; const float* ang; const float2* cs0; const unsigned char* rcode; };
-
-// take pixel q (ticket seen in `m`) for the lane's attempt: 1 taken, 0 it is used after all (committed, or held by a live attempt of
-// lower rank: recorded as a dependency), -1 give up (abortc set)
-__device__ __forceinline__ int ln_take(LaneAtt& A, const LaneFrame& F, int q, unsigned m) {
-    for (int tries = 0; tries < 8; tries++) {
-        const unsigned old = A.mode ? atomicExch(&F.pix[q].used, A.T) : atomicCAS(&F.pix[q].used, m, A.T);
-        if (A.mode || old == m) {
-            const unsigned o = old & 0x7fffffffu;
-            if (o != 0u && o != A.T && v3_classify(o, A.rank, F.rcode) == 3) v3_poison(o);
-            return 1;
-        }
-        m = old;                                                  // somebody changed it in between: look again
-        if (m == A.T) return 0;
-        const int c = m == 0u ? 0 : v3_classify(m, A.rank, F.rcode);
-        if (c == 1) return 0;
-        if (c == 2) {
-            if (!((A.ndeps > 0 && A.dep0 == m) || (A.ndeps > 1 && A.dep1 == m))) { if (A.ndeps == 0) A.dep0 = m; else if (A.ndeps == 1) A.dep1 = m; else { A.abortc = 5; return -1; } A.ndeps++; }
-            return 0;
-        }
-    }
-    A.abortc = 5;                                                 // contended: run it again as head
-    return -1;
-}
-
-// start (or restart, for refine's re-growth) the growth of the lane's attempt from its seed with tolerance prec
-__device__ __forceinline__ void ln_begin(LaneAtt& A, const LaneFrame& F, double prec) {
-    const int sq = (int)A.seedidx;
-    const unsigned m0 = __ldcg(&F.pix[sq].used);
-    if (m0 != A.T) {
-        const int c = m0 == 0u ? 0 : v3_classify(m0, A.rank, F.rcode);
-        if (c == 1) { A.abortc = 4; return; }
-        if (c == 2) { A.abortc = 3; A.conflict = (int)m0; return; }
-        const int t = ln_take(A, F, sq, m0);
-        if (t == 0) { A.abortc = 2; A.conflict = -1; return; }   // lost the seed between the look and the take: look again from the start
-        if (t < 0) return;
-    }
-    A.list[0] = (unsigned)(sq % F.w) | ((unsigned)(sq / F.w) << 16);
-    A.n = 1; A.i = 0; A.kacc = 0;
-    A.th = __ldg(F.ang + sq);
-    const float2 c0 = __ldg(F.cs0 + sq);
-    A.sx = c0.x; A.sy = c0.y; A.rM = rsqrtf(c0.x * c0.x + c0.y * c0.y);
-    A.prec = prec; A.pdeg = (float)(prec * (180.0 / L_PI));
-    A.robok = prec < 0.78;
-    A.coefX = (float)(57.2958 * 1.0002 * sin(prec + 0.17453 + 0.0006));     // vectors accepted within prec + 10 deg of the sums at the last exact angle
-    A.st = LN_GROW;
-}
-
-// one queue entry of the lane's region: the 3x3 scan of lsd.cpp's region_grow, neighbour by neighbour, in order
-__device__ __forceinline__ void ln_step(LaneAtt& A, const LaneFrame& F) {
-    const unsigned pk = A.list[A.i];
-    const int x0 = (int)(pk & 0xffff), y0 = (int)(pk >> 16);
-    uint4 v[8]; int qq[8];
-#pragma unroll
-    for (int j = 0; j < 8; j++) {                                  // the eight records in flight together
-        const int nb = j + (j >= 4 ? 1 : 0);                       // 0..8 without the centre (4)
-        const int xx = x0 + nb % 3 - 1, yy = y0 + nb / 3 - 1;
-        const bool ok = (unsigned)xx < (unsigned)F.w && (unsigned)yy < (unsigned)F.h;
-        qq[j] = ok ? yy * F.w + xx : -1;
-        v[j] = make_uint4(__float_as_uint(NOTDEF_F), 0u, 0u, 0u);
-        if (ok) v[j] = __ldcg(reinterpret_cast<const uint4*>(F.pix + qq[j]));
-    }
-#pragma unroll
-    for (int j = 0; j < 8; j++) {
-        if (A.abortc) break;
-        const float a = __uint_as_float(v[j].x);
-        const unsigned m = v[j].w;
-        if (qq[j] < 0 || a == NOTDEF_F || m == A.T) continue;
-        if (m != 0u) {
-            const int c = v3_classify(m, A.rank, F.rcode);
-            if (c == 1) continue;
-            if (c == 2) {
-                if (!((A.ndeps > 0 && A.dep0 == m) || (A.ndeps > 1 && A.dep1 == m))) { if (A.ndeps == 0) A.dep0 = m; else if (A.ndeps == 1) A.dep1 = m; else { A.abortc = 5; break; } A.ndeps++; }
-                continue;
-            }
-        }
-        // the alignment test against the region angle as the sequential scan has it now
-        bool pass;
-        if (A.kacc == 0) pass = l4_exact_pass<4>(a, A.th, A.pdeg, A.prec);
-        else {
-            const float d = fabsf(A.th - a);
-            const float e = d > 270.f ? 360.f - d : d;
-            const float B = A.coefX * (float)A.kacc * A.rM + 0.0215f;
-            const bool ok = A.robok && B <= 10.f;
-            if (ok && e <= A.pdeg - B) pass = true;
-            else if (ok && e >= A.pdeg + B) pass = false;
-            else {
-                A.th = fast_atan2_deg(A.sy, A.sx); A.rM = rsqrtf(A.sx * A.sx + A.sy * A.sy); A.kacc = 0;
-                pass = l4_exact_pass<4>(a, A.th, A.pdeg, A.prec);
-            }
-        }
-        if (!pass) continue;
-        if (A.n >= A.cap) { A.abortc = 1; break; }
-        const int t = ln_take(A, F, qq[j], m);
-        if (t < 0) break;
-        if (t == 0) continue;
-        const int nb = j + (j >= 4 ? 1 : 0);
-        A.list[A.n++] = (unsigned)(x0 + nb % 3 - 1) | ((unsigned)(y0 + nb / 3 - 1) << 16);
-        A.sx += __uint_as_float(v[j].y); A.sy += __uint_as_float(v[j].z);
-        A.kacc++;
-    }
-    A.i++;
-}
-
-__global__ void __launch_bounds__(32, 8) k_lsd_regions_lanes(const __grid_constant__ LineGeom g, LineWs ws, int nframes) {
-    constexpr int SOLO = 4;
-    V3Shared& S = v3s();
-    const int lane = threadIdx.x;
-    const unsigned lt = (1u << lane) - 1u;
-  for (;;) {
-    __syncwarp();
-    if (lane == 0) {
-        const int f = atomicAdd(ws.rejctl + 2, 1);
-        S.frame = f; S.turn = 0; S.nclaims = 0; S.cursor = 0; S.nj = 0; S.all_claimed = 0; S.done = 0; S.nready = 0; S.nblocked = 0; S.dl_used = 0; S.scanhint = 0; S.win_base = -(1 << 30); S.overflow = 0;
-        S.ns = f < nframes ? ws.nseeds[f] : 0;
-    }
-    for (int i = lane; i < V3_RING; i += 32) { S.state[i] = V3_EMPTY; S.wait[i] = -1; S.tryno[i] = 0; S.poison[i] = 0; S.flag[i] = 0; S.dl_n[i] = 0; }
-    for (int i = lane; i < V3_RANKS / 32; i += 32) S.excbits[i] = 0u;
-    __syncwarp();
-    const int f = S.frame;
-    if (f >= nframes) break;
-    unsigned char* rcode = ws.rcode + (long long)f * V3_RANKS;
-    LaneFrame F; F.w = g.sw; F.h = g.sh; F.pix = ws.pix + f * g.pix_stride; F.ang = ws.angdeg + f * g.pix_stride; F.cs0 = ws.cs0 + f * g.pix_stride; F.rcode = rcode;
-    if (lane == 0) {
-        WalkCtx& W = s_W1;
-        W.w = g.sw; W.h = g.sh; W.dbg = g.dbg;
-        W.ang = F.ang; W.mod = ws.modgrad + f * g.pix_stride; W.pix = F.pix; W.cs0 = F.cs0; W.bits = reinterpret_cast<const unsigned*>(rcode);
-    }
-    __syncwarp();
-    unsigned* const mylist = ws.sreg + ((long long)f * 32 + lane) * LN_LIST;
-    unsigned* const biglist = ws.reg + (long long)f * g.pix_stride;
-    LaneAtt A; A.st = LN_IDLE; A.abortc = 0; A.ndeps = 0; A.dep0 = A.dep1 = 0u; A.n = 0; A.i = 0; A.kacc = 0; A.mode = 0; A.phase = 0; A.dirty = 0; A.acc = 0; A.n0 = 0;
-    A.slot = 0; A.rank = 0; A.tryno = 0; A.T = 0u; A.list = mylist; A.cap = LN_LIST; A.sx = A.sy = A.th = A.rM = A.pdeg = A.coefX = 0.f; A.prec = 0; A.robok = 0; A.conflict = -1; A.seedidx = 0u;
-    unsigned long long dummy[6] = {0, 0, 0, 0, 0, 0};
-    const bool stat = (g.dbg & 32) != 0;
-    unsigned long long c_ret = 0, c_asg = 0, c_grow = 0, c_post = 0, n_iter = 0, n_round = 0, n_act = 0, n_post = 0;
-    for (;;) {
-        const long long q0 = stat ? clock64() : 0;
-        // ---- retire the head of the ring while it is finished (the whole warp, cooperatively)
-        {
-            const unsigned t = S.turn;
-            const int hs = t < S.nclaims ? *reinterpret_cast<volatile int*>(&S.state[t & (V3_RING - 1)]) : V3_EMPTY;
-            if (hs == V3_DONE || hs == V3_PRESUMED || hs == V3_VOID) v3_retire_pass(g, ws, f, rcode, dummy);
-        }
-        if (S.all_claimed && S.turn >= S.nclaims) break;
-        const long long q1 = stat ? clock64() : 0;
-        // ---- finished lanes that need no cooperative work publish their own slot: regions below the minimum size, and every abort
-        if (A.st == LN_POST && (A.abortc || (A.phase == 0 && A.n < g.min_reg_size))) {
-            const int slot = A.slot, y = A.tryno;
-            if (!A.abortc) {
-                S.dep[slot][0] = A.dep0; S.dep[slot][1] = A.dep1; S.dl_n[slot] = 0;
-                S.flag[slot] = (unsigned char)(V3F_RAN | (A.ndeps << 4));
-                __threadfence_block();
-                *reinterpret_cast<volatile int*>(&S.state[slot]) = V3_DONE;
-            } else if (A.abortc == 4) { S.tryno[slot] = (unsigned char)min(y + 1, 126); S.flag[slot] = V3F_RAN; __threadfence_block(); *reinterpret_cast<volatile int*>(&S.state[slot]) = V3_VOID; }
-            else if (A.abortc == 3) { S.tryno[slot] = (unsigned char)min(y + 1, 126); S.poison[slot] = 0; S.flag[slot] = V3F_RAN; S.dep[slot][0] = (unsigned)A.conflict; __threadfence_block(); *reinterpret_cast<volatile int*>(&S.state[slot]) = V3_PRESUMED; }
-            else {
-                S.tryno[slot] = (unsigned char)min(y + 1, 126); S.poison[slot] = 0; S.flag[slot] = V3F_RAN;
-                int wt = A.abortc == 2 ? A.conflict : A.rank;
-                if (y >= 100) wt = A.rank;
-                S.wait[slot] = wt;
-                if (wt >= 0) atomicAdd(&S.nblocked, 1);
-                atomicMin(&S.scanhint, A.rank);
-                __threadfence_block();
-                atomicAdd(&S.nready, 1);
-                *reinterpret_cast<volatile int*>(&S.state[slot]) = V3_READY;
-            }
-            A.st = LN_IDLE; A.abortc = 0;
-        }
-        __syncwarp();
-        const unsigned idle = __ballot_sync(0xffffffffu, A.st == LN_IDLE);
-        if (idle) {
-            for (int pass = 0; pass < 3 && !S.all_claimed && *reinterpret_cast<volatile int*>(&S.nready) - *reinterpret_cast<volatile int*>(&S.nblocked) < __popc(idle) + 8; pass++)
-                if (!v3_claim_pass(g, ws, f, rcode, 1 << 20)) break;
-            // ---- hand runnable slots to the idle lanes, lowest ranks first
-            const unsigned t = S.turn, nc = S.nclaims;
-            int from = max((int)t, *reinterpret_cast<volatile int*>(&S.scanhint));
-            unsigned left = idle;
-            bool sawready = false;
-            for (int b = from; b < (int)nc && left; b += 32) {
-                const int r = b + lane;
-                bool ready = false, run = false;
-                if (r < (int)nc) {
-                    const int k = r & (V3_RING - 1);
-                    ready = *reinterpret_cast<volatile int*>(&S.state[k]) == V3_READY;
-                    if (ready) {
-                        const int wt = *reinterpret_cast<volatile int*>(&S.wait[k]);
-                        if (wt == r) run = r == (int)t;
-                        else { run = wt < (int)t; if (!run) { const int sw = *reinterpret_cast<volatile int*>(&S.state[wt & (V3_RING - 1)]); run = sw != V3_READY && sw != V3_RUNNING; } }
-                    }
-                }
-                const unsigned rm = __ballot_sync(0xffffffffu, run);
-                if (!sawready) { if (__ballot_sync(0xffffffffu, ready)) sawready = true; else if (lane == 0 && b == from && b + 32 <= (int)nc) atomicCAS(&S.scanhint, from, b + 32); }
-                // the j-th idle lane takes the j-th runnable slot of this block
-                const int take = min(__popc(rm), __popc(left));
-                if (take) {
-                    const bool mine = ((left >> lane) & 1u) && __popc(left & lt) < take;
-                    if (mine) {
-                        const int r0 = b + (int)__fns(rm, 0, __popc(left & lt) + 1);
-                        const int k = r0 & (V3_RING - 1);
-                        *reinterpret_cast<volatile int*>(&S.state[k]) = V3_RUNNING;       // one warp per frame: nobody competes for the slot
-                        atomicSub(&S.nready, 1);
-                        if (S.wait[k] >= 0) atomicSub(&S.nblocked, 1);
-                        A.slot = k; A.rank = r0; A.tryno = S.tryno[k]; A.seedidx = (unsigned)S.seed[k];
-                        A.T = (unsigned)(r0 + 1) | ((unsigned)A.tryno << 24);
-                        A.mode = r0 == (int)t ? 1 : 0;
-                        A.list = A.mode ? biglist : mylist; A.cap = A.mode ? (int)g.pix_stride : LN_LIST;
-                        A.phase = 0; A.abortc = 0; A.conflict = -1; A.ndeps = 0; A.dirty = 0; A.acc = 0; A.n0 = 0; A.n = 0; A.i = 0;
-                        ln_begin(A, F, g.prec);
-                        if (A.abortc) A.st = LN_POST;              // (settled at the top of the next iteration)
-                    }
-                    left &= ~__ballot_sync(0xffffffffu, mine);
-                }
-            }
-        }
-        const long long q2 = stat ? clock64() : 0;
-        // ---- growth: every busy lane expands one queue entry of its own region
-        {
-            if (stat) { n_round++; n_act += __popc(__ballot_sync(0xffffffffu, A.st == LN_GROW)); }
-            if (A.st == LN_GROW) {
-                if (A.mode == 0 && *reinterpret_cast<volatile unsigned char*>(&S.poison[A.slot]) == (unsigned char)(A.tryno + 1)) { A.abortc = 2; A.conflict = -1; }
-                if (!A.abortc && A.i < A.n) ln_step(A, F);
-                if (A.abortc || A.i >= A.n) A.st = LN_POST;
-            }
-            __syncwarp();
-        }
-        const long long q3 = stat ? clock64() : 0;
-        if (stat) { c_ret += q1 - q0; c_asg += q2 - q1; c_grow += q3 - q2; n_iter++; }
-        // ---- post: one finished lane at a time, the warp works on its region together (lowest rank first)
-        for (;;) {
-            const bool coop = A.st == LN_POST && !A.abortc && !(A.phase == 0 && A.n < g.min_reg_size);
-            const unsigned pm = __ballot_sync(0xffffffffu, coop);
-            if (!pm) { if (stat) c_post += clock64() - q3; break; }
-            n_post++;
-            int best = coop ? A.rank : 0x7fffffff;
-            best = __reduce_min_sync(0xffffffffu, best);
-            const int L = __ffs(__ballot_sync(0xffffffffu, coop && A.rank == best)) - 1;
-            // the lane's attempt, broadcast
-            const int abortc = __shfl_sync(0xffffffffu, A.abortc, L), slot = __shfl_sync(0xffffffffu, A.slot, L), rank = __shfl_sync(0xffffffffu, A.rank, L);
-            const int mode = __shfl_sync(0xffffffffu, A.mode, L), phase = __shfl_sync(0xffffffffu, A.phase, L), tryno = __shfl_sync(0xffffffffu, A.tryno, L);
-            int n = __shfl_sync(0xffffffffu, A.n, L);
-            const unsigned long long lp = __shfl_sync(0xffffffffu, (unsigned long long)A.list, L);
-            unsigned* list = reinterpret_cast<unsigned*>(lp);
-            const int cap = __shfl_sync(0xffffffffu, A.cap, L);
-            const unsigned T = __shfl_sync(0xffffffffu, A.T, L), seedidx = __shfl_sync(0xffffffffu, A.seedidx, L);
-            int res = -1;            // -1 aborted, 0 no job, 1 job, 2 keeps growing (re-growth started)
-            LRect rec;
-            if (!abortc) {
-                // region angle at the end of the growth: exact
-                float th = __shfl_sync(0xffffffffu, A.th, L);
-                { const float sx = __shfl_sync(0xffffffffu, A.sx, L), sy = __shfl_sync(0xffffffffu, A.sy, L); if (__shfl_sync(0xffffffffu, A.kacc, L) > 0) th = fast_atan2_deg(sy, sx); }
-                double reg_angle = (double)th * L_DEG;
-                __syncwarp();
-                if (lane == 0) { WalkCtx& W = s_W1; W.reg = list; W.base0 = mode ? biglist : (ws.sreg + ((long long)f * 32 + L) * LN_LIST); W.cap = cap; W.mode = mode; W.ticket = T; W.seq = rank; W.abort = 0; W.dirty = 0; W.nasm = 0; }
-                __syncwarp();
-                int n0 = __shfl_sync(0xffffffffu, A.n0, L), acc = __shfl_sync(0xffffffffu, A.acc, L);
-                if (phase == 0) {
-                    n0 = n; acc = n;
-                    if (lane == 0) s_W1.acc = acc;
-                    __syncwarp();
-                    if (n < g.min_reg_size) res = 0;
-                    else {
-                        l_region2rect<SOLO>(n, reg_angle, g.prec, g.p, &rec);
-                        double tau;
-                        if (l4_refine_begin(n, &rec, 0.7, &tau)) res = 1;
-                        else {
-                            // re-growth from the seed with tolerance tau: the lane goes back to growing (behind its first list if speculative)
-                            if (lane == L) {
-                                A.dirty = 1; A.phase = 1; A.n0 = n0; A.acc = acc;
-                                if (mode == 0) { A.list += n; A.cap -= n; }
-                                if (A.cap < 8) A.abortc = 1; else ln_begin(A, F, tau);
-                                if (A.abortc) A.st = LN_POST;         // settled in the next round of this loop
-                            }
-                            res = 2;
-                        }
-                    }
-                } else {
-                    if (mode == 0) acc += n;
-                    if (lane == 0) { s_W1.acc = acc; s_W1.dirty = 1; }
-                    __syncwarp();
-                    if (n < 2) res = 0;
-                    else {
-                        l_region2rect<SOLO>(n, reg_angle, g.prec, g.p, &rec);
-                        const double density = (double)n / (l_dist(rec.x1, rec.y1, rec.x2, rec.y2) * rec.width);
-                        bool okr = true;
-                        if (density < 0.7) { int nn = n; okr = l_reduce_region_radius<SOLO>(&nn, reg_angle, g.prec, g.p, &rec, density, 0.7); if (s_W1.abort) okr = false; }
-                        res = s_W1.abort ? -1 : (okr ? 1 : 0);
-                    }
-                }
-                __syncwarp();
-                if (res == 2) continue;
-                // publish
-                const int dirty = phase == 1 ? 1 : 0;
-                int res2 = res;
-                if (res >= 0 && dirty && mode == 0) {
-                    int off = 0;
-                    if (lane == 0) off = atomicAdd(&S.dl_used, acc);
-                    off = __shfl_sync(0xffffffffu, off, 0);
-                    if (off + acc > V3_DPOOL) res2 = -2;
-                    else {
-                        unsigned* dst = ws.dlist + (long long)f * V3_DPOOL + off;
-                        const unsigned* src = ws.sreg + ((long long)f * 32 + L) * LN_LIST;
-                        for (int i = lane; i < acc; i += 32) dst[i] = src[i];
-                        if (lane == 0) { S.dl_off[slot] = off; S.dl_n[slot] = acc; }
-                    }
-                } else if (lane == 0) S.dl_n[slot] = 0;
-                __syncwarp();
-                if (res2 >= 0) {
-                    if (res == 1) l_emit_job(g, ws.sjob + ((long long)f * V3_RING + slot) * 13, rec, seedidx, n0, lane);
-                    __syncwarp();
-                    const int nd = __shfl_sync(0xffffffffu, A.ndeps, L);
-                    const unsigned d0 = __shfl_sync(0xffffffffu, A.dep0, L), d1 = __shfl_sync(0xffffffffu, A.dep1, L);
-                    if (lane == 0) {
-                        S.dep[slot][0] = d0; S.dep[slot][1] = d1;
-                        S.flag[slot] = (unsigned char)(V3F_RAN | (res == 1 ? V3F_JOB : 0) | (dirty ? V3F_DIRTY : 0) | (nd << 4));
-                        __threadfence();
-                        *reinterpret_cast<volatile int*>(&S.state[slot]) = V3_DONE;
-                    }
-                    __syncwarp();
-                    if (lane == L) A.st = LN_IDLE;
-                    continue;
-                }
-            }
-            // aborted (by the growth, by the cooperative part, or no room for its released-pixel list)
-            {
-                int ab = abortc ? abortc : (res == -1 ? (s_W1.abort ? s_W1.abort : 1) : 1);
-                const int conflict = __shfl_sync(0xffffffffu, A.conflict, L);
-                if (lane == 0) {
-                    const int y = tryno;
-                    if (ab == 4) { S.tryno[slot] = (unsigned char)min(y + 1, 126); S.flag[slot] = V3F_RAN; __threadfence_block(); *reinterpret_cast<volatile int*>(&S.state[slot]) = V3_VOID; }
-                    else if (ab == 3) { S.tryno[slot] = (unsigned char)min(y + 1, 126); S.poison[slot] = 0; S.flag[slot] = V3F_RAN; S.dep[slot][0] = (unsigned)conflict; __threadfence_block(); *reinterpret_cast<volatile int*>(&S.state[slot]) = V3_PRESUMED; }
-                    else {
-                        S.tryno[slot] = (unsigned char)min(y + 1, 126); S.poison[slot] = 0; S.flag[slot] = V3F_RAN;
-                        int wt = ab == 2 ? conflict : rank;
-                        if (y >= 100) wt = rank;
-                        S.wait[slot] = wt;
-                        if (wt >= 0) atomicAdd(&S.nblocked, 1);
-                        atomicMin(&S.scanhint, rank);
-                        __threadfence_block();
-                        atomicAdd(&S.nready, 1);
-                        *reinterpret_cast<volatile int*>(&S.state[slot]) = V3_READY;
-                    }
-                }
-                __syncwarp();
-                if (lane == L) { A.st = LN_IDLE; A.abortc = 0; }
-            }
-        }
-    }
-    __syncwarp();
-    if (stat && lane == 0) {
-        atomicAdd(ws.wstat + 0, n_iter); atomicAdd(ws.wstat + 1, n_round); atomicAdd(ws.wstat + 2, n_act); atomicAdd(ws.wstat + 3, n_post);
-        atomicAdd(ws.wstat + 8, c_ret); atomicAdd(ws.wstat + 9, c_asg); atomicAdd(ws.wstat + 10, c_grow); atomicAdd(ws.wstat + 11, c_post); atomicAdd(ws.wstat + 13, (unsigned long long)S.nclaims);
-    }
-    if (lane == 0) { ws.njobs[f] = min(S.nj, g.seg_cap); if (S.nj > g.seg_cap || S.overflow) atomicOr(ws.err, DERR_LSD_OVERFLOW); }
-  }
-}
-
 // NFA of every candidate region of every frame, in three data-parallel steps (grids are sized by the work, not by the
 // per-frame capacity seg_cap, which is ~13k slots of which a few hundred are used):
 //   k_lsd_nfa_count   one warp per job: the rectangle scan (total / aligned pixel counts)
@@ -2832,11 +1657,7 @@ struct sslpl_line {
     int used_smem = 0;
     int sm_count = 148;
     int max_walkers = 0;        // 0 = one walker CTA per frame
-    int walker_warps = 0;       // 0 = automatic (8 or 16 warps per frame)
-    int walker_v3 = 0;          // multi-warp walker: 0 = the round-2a form (shipped), 1 = v3 (control warps + workers, O(1) retire), -1 = v3 by frame size
-    int used_smem3 = 0, used_smem4 = 0;
-    int walker_lanes = 0;       // one warp per frame, lane-parallel region growing (SSLPL_WALKER_LANES=1)
-    int walker_lean = 0;        // one-warp walker: 0 = the round-2a form (shipped: faster when several launches overlap), 1 = lean region growing (SSLPL_WALKER_LEAN=1)
+    int walker_warps = 0;       // 0 = automatic (one warp or 16 warps per frame), -1 = one warp
     int cur_w = 0, cur_h = 0, cur_frames = 0;
     long long launches = 0;
     int* h_err = nullptr;
@@ -2873,7 +1694,6 @@ void make_geometry(const sslpl_line* h, int W, int H, LineGeom& g, std::vector<i
     g.seg_cap = (int)(g.pix_stride / std::max(g.min_reg_size, 1)) + 16;
     g.trace_cap = h->trace ? g.seg_cap : 0;
     g.dbg = getenv("SSLPL_WALKER_DBG") ? atoi(getenv("SSLPL_WALKER_DBG")) : 0;
-    g.dbg_seed = getenv("SSLPL_WALKER_SEED") ? atoi(getenv("SSLPL_WALKER_SEED")) : -1;
     if (tab) {
         tab->assign(g.sw + g.sh, make_int2(0, 0));
         for (int axis = 0; axis < 2; axis++) {
@@ -2902,7 +1722,7 @@ void carve(sslpl_line* h, Arena& A, const LineGeom& g, int B) {
     ws.maxgrad = A.take<unsigned long long>(B);
     ws.seeds = A.take<unsigned>((size_t)B * g.pix_stride); ws.nseeds = A.take<int>(B);
     ws.reg = A.take<unsigned>((size_t)B * g.pix_stride);
-    ws.sreg = A.take<unsigned>((size_t)B * WALK_RING * WALK_SLOT_CAP); ws.sjob = A.take<double>((size_t)B * V3_RING * 13); ws.rcode = A.take<unsigned char>((size_t)B * V3_RANKS); ws.dlist = A.take<unsigned>((size_t)B * V3_DPOOL);
+    ws.sreg = A.take<unsigned>((size_t)B * WALK_RING * WALK_SLOT_CAP);
     ws.wstat = A.take<unsigned long long>(16);
     ws.seg = A.take<double>((size_t)B * g.seg_cap * 4); ws.nseg = A.take<int>(B);
     ws.jobs = A.take<double>((size_t)B * g.seg_cap * 13); ws.njobs = A.take<int>(B); ws.jobflag = A.take<int>((size_t)B * g.seg_cap);
@@ -2968,28 +1788,14 @@ int run_pipeline(sslpl_line* h, int B) {
     SSLPL_CUDA(cudaMemsetAsync(h->ws.rejctl, 0, 4 * sizeof(int), st));
     SSLPL_CUDA(cudaMemsetAsync(h->ws.wstat, 0, 16 * sizeof(unsigned long long), st));
     {   // one CTA per frame; few frames -> more warps per frame (latency), many frames -> more CTAs per SM (throughput)
-        // automatic choice (measured, B200): big batches -> one warp per frame (throughput); one or a few frames -> a multi-warp CTA per
-        // frame, the round-2a walker with 16 warps.  v3 (SSLPL_WALKER_V3=1, 8 warps) is level with it on 640x480 frames (15.0-17.0 ms over
-        // runs against 17.2 ms) and behind on 1280x960 (115 ms against 69 ms: its deeper speculation loses more work than it overlaps), so
-        // it is not the default; SSLPL_WALKER_V3=-1 picks it by frame size (up to ~0.3 M detection-scale pixels)
-        const bool small = g.pix_stride <= 300000;
-        const bool v3 = h->walker_v3 > 0 || (h->walker_v3 < 0 && small);
-        const int ww = h->walker_warps < 0 ? 0 : h->walker_warps > 0 ? std::min(h->walker_warps, WALK_MAXW) : (B >= 2 * h->sm_count ? 0 : (v3 ? 8 : WALK_MAXW));
+        // automatic choice (measured, B200): big batches (at least two frames per SM) -> one warp per frame (k_lsd_regions_solo);
+        // fewer frames -> the multi-warp walker k_lsd_regions with 16 warps per frame.  SSLPL_WALKER_WARPS overrides it (-1 = one warp).
+        const int ww = h->walker_warps < 0 ? 0 : h->walker_warps > 0 ? std::min(h->walker_warps, WALK_MAXW) : (B >= 2 * h->sm_count ? 0 : WALK_MAXW);
         const size_t smem = (size_t)((g.pix_stride + 31) / 32) * sizeof(unsigned);
         if ((int)smem > h->used_smem) { SSLPL_CUDA(cudaFuncSetAttribute(k_lsd_regions, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); h->used_smem = (int)smem; }
-        if (h->walker_lanes && ww == 0) {
-            const size_t sm4 = sizeof(V3Shared);
-            if ((int)sm4 > h->used_smem4) { SSLPL_CUDA(cudaFuncSetAttribute(k_lsd_regions_lanes, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm4)); h->used_smem4 = (int)sm4; }
-            k_lsd_regions_lanes<<<(h->max_walkers > 0 ? std::min(B, h->max_walkers) : B), 32, sm4, st>>>(g, h->ws, B);
-        }
-        else if (ww >= 2 && v3) {
-            const size_t sm3 = sizeof(V3Shared) + (size_t)ww * V3_LRING * sizeof(unsigned);
-            if ((int)sm3 > h->used_smem3) { SSLPL_CUDA(cudaFuncSetAttribute(k_lsd_regions_v3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm3)); h->used_smem3 = (int)sm3; }
-            k_lsd_regions_v3<<<(h->max_walkers > 0 ? std::min(B, h->max_walkers) : B), ww * 32, sm3, st>>>(g, h->ws, B);
-        }
-        else if (ww == 0 && h->walker_lean) k_lsd_regions_lean<<<(h->max_walkers > 0 ? std::min(B, h->max_walkers) : B), 32, 0, st>>>(g, h->ws, B);   // one warp per frame
-        else if (ww == 0) k_lsd_regions_solo<<<(h->max_walkers > 0 ? std::min(B, h->max_walkers) : B), 32, 0, st>>>(g, h->ws, B);              // round-2a form (A/B)
-        else k_lsd_regions<<<(h->max_walkers > 0 ? std::min(B, h->max_walkers) : B), ww * 32, smem, st>>>(g, h->ws, B);
+        const int grid = h->max_walkers > 0 ? std::min(B, h->max_walkers) : B;
+        if (ww == 0) k_lsd_regions_solo<<<grid, 32, 0, st>>>(g, h->ws, B);
+        else k_lsd_regions<<<grid, ww * 32, smem, st>>>(g, h->ws, B);
     }
     lmark(h, "lsd_regions");
     k_lsd_nfa_count<<<dim3(NFA_COUNT_CTAS, B), 128, 0, st>>>(g, h->ws);
@@ -3032,9 +1838,6 @@ int sslpl_line_create(const sslpl_line_params* p, sslpl_line** out) {
     h->p = *p;
     { int v = 0; if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, p->device) == cudaSuccess && v > 0) h->sm_count = v; }
     h->trace = getenv("SSLPL_LINE_TRACE") != nullptr;
-    if (const char* e = getenv("SSLPL_WALKER_LANES")) h->walker_lanes = atoi(e) != 0;
-    if (const char* e = getenv("SSLPL_WALKER_V3")) h->walker_v3 = atoi(e) < 0 ? -1 : (atoi(e) != 0 ? 1 : 0);
-    if (const char* e = getenv("SSLPL_WALKER_LEAN")) h->walker_lean = atoi(e) != 0;
     if (const char* e = getenv("SSLPL_WALKER_WARPS")) h->walker_warps = std::max(-1, std::min(WALK_MAXW, atoi(e)));   // tuning knob (tests sweep it); -1 = the one-warp throughput kernel
     {   // BinaryDescriptor constructor: local (F_l) and global (F_g) Gaussian weights, widthOfBand 7, 9 bands
         double u = (7 * 3 - 1) / 2, sigma = (7 * 2 + 1) / 2, inv = -1 / (2 * sigma * sigma);
@@ -3168,13 +1971,11 @@ int sslpl_line_download_segments(sslpl_line* h, int frame, float* seg4, int cap,
 
 
 /* debug (SSLPL_LINE_TRACE=1 at handle creation): one row of 10 doubles per region that reached region2rect */
-/* Statistics of the last region-walker launch (16 values; collected with SSLPL_WALKER_DBG=32).  For the round-2a multi-warp walker as
-   listed below; the v3 and lane-parallel walkers fill the same array with their own counters (tools/v3_stats.py, tools/lanes_stats.py
-   name them).  Round-2a: [0] regions grown by the turn holder, [1] their clock cycles, [2] their
-   pixels, [3] -, [4] claims whose seed had been swallowed by commit time, [5] redone by the turn holder: abandoned, [6] poisoned,
-   [7] failed validation, [8] presumed swallowed but not, [9] attempts committed as speculated, [10] their pixels, [11] cycles
-   under the commit lock, [12] under the claim lock, [13] attempts repeated after a lower rank retired, [14] cycles per frame
-   (summed), [15] claims. */
+/* Statistics of the last region-walker launch (16 values; collected with SSLPL_WALKER_DBG=32 by the multi-warp walker k_lsd_regions):
+   [0] regions grown by the turn holder, [1] their clock cycles, [2] their pixels, [3] -, [4] claims whose seed had been swallowed
+   by commit time, [5] redone by the turn holder: abandoned, [6] poisoned, [7] failed validation, [8] presumed swallowed but not,
+   [9] attempts committed as speculated, [10] their pixels, [11] cycles under the commit lock, [12] under the claim lock, [13] attempts
+   repeated after a lower rank retired, [14] cycles per frame (summed), [15] claims. */
 int sslpl_line_walker_stats(sslpl_line* h, unsigned long long* out16) {
     SSLPL_REQUIRE(h && out16, SSLPL_ERR_ARG, "null argument");
     SSLPL_CUDA(cudaSetDevice(h->p.device));

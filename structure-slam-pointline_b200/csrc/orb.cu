@@ -63,8 +63,6 @@ struct OrbWs {
 
 struct View { const uint8_t* base; int pitch; long long frame_stride; };
 
-struct TMaps { CUtensorMap lvl[MAXL]; CUtensorMap pyr[MAXL]; };     // per pyramid level: 3-D (x, y, frame) u8 tensor maps with the 96x38 box of the stencil kernels and with the 128x32 box of k_pyr2
-
 __constant__ signed char c_pattern[1024] = {
 #include "orb_pattern.inc"
 };
@@ -216,115 +214,6 @@ __device__ __forceinline__ void stage_box(uint8_t* s_img, uint64_t* s_bar, const
             }
         }
         __syncthreads();
-    }
-}
-
-// TWO pyramid levels per launch (round 2b): the CTA owns a 64x16 tile of level L+1, stages the box of level L-1 that it depends on
-// (one TMA bulk copy; 128x32 covers 64 * 1.2^2 + the 16-byte alignment slack), computes the region of level L behind its tile into
-// shared memory — writing out the part it OWNS (the level-L columns / rows from its first source index up to the next tile's) — and
-// from that its tile of level L+1.  Neighbouring CTAs recompute the one-pixel halo of level L (about 30 % more level-L arithmetic;
-// level L-1 is read once, level L is never read back).  Same fixed-point arithmetic and tables as k_resize, so the planes are
-// bit-identical.  The host falls back to k_resize for a level pair whose spans exceed the tiles below (never at scale 1.2) and for
-// the last level when their number is odd.  MEASURED (513 frames 640x480): 1.00 ms against 0.85 ms for the seven k_resize launches —
-// the plain kernel's byte loads already hit L1 / L2, while a 64x16 tile pays one TMA round trip and 30 % recomputed halo; it is kept
-// behind SSLPL_PYR2=1 (tests/test_orb_gpu.py::test_pyramid_two_levels_per_launch_path), k_resize stays the default.
-constexpr int PY_TW = 64, PY_TH = 16, PY_MP = 88, PY_MH = 24, PY_BW = 128, PY_BH = 32;
-
-__device__ __forceinline__ int resize_px(int p00, int p01, int p10, int p11, int a0, int a1, int b0, int b1) {
-    const int r0 = p00 * a0 + p01 * a1, r1 = p10 * a0 + p11 * a1;
-    return (((b0 * (r0 >> 4)) >> 16) + ((b1 * (r1 >> 4)) >> 16) + 2) >> 2;
-}
-
-template <bool TMA>
-__global__ void __launch_bounds__(256) k_pyr2(const __grid_constant__ OrbGeom g, OrbWs ws, View v, const CUtensorMap* tm, int L) {
-    __shared__ __align__(128) uint8_t s_box[PY_BW * PY_BH];
-    __shared__ __align__(16) uint8_t s_mid[PY_MP * PY_MH];
-    __shared__ uint64_t s_bar;
-    const LevelGeom& S = g.lv[L - 1]; const LevelGeom& M = g.lv[L]; const LevelGeom& U = g.lv[L + 1];
-    const int tid = threadIdx.x, f = blockIdx.z;
-    const int ux0 = blockIdx.x * PY_TW, uy0 = blockIdx.y * PY_TH;
-    const int ux1 = min(ux0 + PY_TW, U.w), uy1 = min(uy0 + PY_TH, U.h);                    // exclusive
-    const int2* __restrict__ xtU = ws.rtab + U.xtab_off; const int2* __restrict__ ytU = ws.rtab + U.ytab_off;
-    const int2* __restrict__ xtM = ws.rtab + M.xtab_off; const int2* __restrict__ ytM = ws.rtab + M.ytab_off;
-    const bool lastx = ux1 == U.w, lasty = uy1 == U.h;
-    const int cx0 = __ldg(&xtU[ux0]).x, cy0 = __ldg(&ytU[uy0]).x;                          // level-L region behind the tile (inclusive)
-    const int cx1 = lastx ? M.w - 1 : min(__ldg(&xtU[ux1 - 1]).x + 1, M.w - 1);
-    const int cy1 = lasty ? M.h - 1 : min(__ldg(&ytU[uy1 - 1]).x + 1, M.h - 1);
-    const int ox1 = lastx ? M.w : __ldg(&xtU[ux1]).x, oy1 = lasty ? M.h : __ldg(&ytU[uy1]).x;   // owned part: [cx0, ox1) x [cy0, oy1)
-    const int qx0 = cx0 & ~3;                                                              // s_mid columns start at a multiple of 4 of level L
-    const int bx0 = __ldg(&xtM[cx0]).x, by0 = __ldg(&ytM[cy0]).x, ax0 = bx0 & ~15;         // staged box of level L-1: origin (ax0, by0)
-    int sp;
-    const uint8_t* src = level_ptr(g, ws, v, L - 1, f, &sp);
-    if (TMA) {
-        if (tid == 0) mbar_init(&s_bar, 1);
-        __syncthreads();
-        if (tid == 0) {
-            asm volatile("fence.proxy.tensormap::generic.acquire.gpu [%0], 128;" ::"l"(reinterpret_cast<uint64_t>(tm + MAXL + L - 1)) : "memory");
-            mbar_expect_tx(&s_bar, PY_BW * PY_BH);
-            tma_load_3d(s_box, tm + MAXL + L - 1, ax0, by0, f, &s_bar);
-        }
-        mbar_wait(&s_bar, 0);
-    } else {
-        for (int i = tid; i < PY_BW * PY_BH; i += 256) {
-            const int r = i / PY_BW, c = i - r * PY_BW;
-            s_box[i] = __ldg(src + (long long)min(by0 + r, S.h - 1) * sp + min(ax0 + c, S.w - 1));
-        }
-        __syncthreads();
-    }
-    // ---- level L: the region [qx0 .. cx1] x [cy0 .. cy1] in quads of 4 columns
-    int mp;
-    uint8_t* Mg = const_cast<uint8_t*>(level_ptr(g, ws, v, L, f, &mp));
-    const int nq = (cx1 - qx0) / 4 + 1, nr = cy1 - cy0 + 1;
-    for (int i = tid; i < nq * nr; i += 256) {
-        const int r = i / nq, x4 = qx0 + (i - r * nq) * 4, y = cy0 + r;
-        const int2 ty = __ldg(&ytM[y]);
-        const int b0 = ty.y & 0xffff, b1 = ty.y >> 16;
-        const uint8_t* R0 = s_box + (ty.x - by0) * PY_BW - ax0;
-        const uint8_t* R1 = s_box + (min(ty.x + 1, S.h - 1) - by0) * PY_BW - ax0;
-        uint32_t out = 0;
-#pragma unroll
-        for (int k = 0; k < 4; k++) {
-            const int x = x4 + k;
-            if (x >= cx0 && x <= cx1) {
-                const int2 tx = __ldg(&xtM[x]);
-                const int sx = tx.x, sx1 = min(sx + 1, S.w - 1);
-                const int o = resize_px(R0[sx], R0[sx1], R1[sx], R1[sx1], tx.y & 0xffff, tx.y >> 16, b0, b1);
-                out |= (uint32_t)(o & 255) << (8 * k);
-            }
-        }
-        *reinterpret_cast<uint32_t*>(s_mid + r * PY_MP + (x4 - qx0)) = out;
-        if (y < oy1) {
-            uint8_t* dst = Mg + (long long)y * mp + x4;
-            if (x4 >= cx0 && x4 + 3 < ox1) *reinterpret_cast<uint32_t*>(dst) = out;         // pitch and x4 are multiples of 4
-            else for (int k = 0; k < 4; k++) if (x4 + k >= cx0 && x4 + k < ox1) dst[k] = (uint8_t)(out >> (8 * k));
-        }
-    }
-    __syncthreads();
-    // ---- level L+1: the tile, 4 pixels per thread
-    {
-        const int x4 = ux0 + (tid & 15) * 4, y = uy0 + (tid >> 4);
-        if (y < uy1 && x4 < ux1) {
-            int up;
-            uint8_t* Ug = const_cast<uint8_t*>(level_ptr(g, ws, v, L + 1, f, &up));
-            const int2 ty = __ldg(&ytU[y]);
-            const int b0 = ty.y & 0xffff, b1 = ty.y >> 16;
-            const uint8_t* R0 = s_mid + (ty.x - cy0) * PY_MP - qx0;
-            const uint8_t* R1 = s_mid + (min(ty.x + 1, M.h - 1) - cy0) * PY_MP - qx0;
-            uint32_t out = 0;
-#pragma unroll
-            for (int k = 0; k < 4; k++) {
-                const int x = x4 + k;
-                if (x < ux1) {
-                    const int2 tx = __ldg(&xtU[x]);
-                    const int sx = tx.x, sx1 = min(sx + 1, M.w - 1);
-                    const int o = resize_px(R0[sx], R0[sx1], R1[sx], R1[sx1], tx.y & 0xffff, tx.y >> 16, b0, b1);
-                    out |= (uint32_t)(o & 255) << (8 * k);
-                }
-            }
-            uint8_t* dst = Ug + (long long)y * up + x4;
-            if (x4 + 3 < U.w) *reinterpret_cast<uint32_t*>(dst) = out;
-            else for (int k = 0; x4 + k < U.w; k++) dst[k] = (uint8_t)(out >> (8 * k));
-        }
     }
 }
 
@@ -906,11 +795,10 @@ struct sslpl_orb {
     std::vector<cudaEvent_t> ev; std::vector<const char*> ev_name; int ev_n = 0;
     int* h_err = nullptr;               // pinned
     int octree_smem = 0;
-    TMaps tm;                           // per-level tensor maps (level 0 re-encoded per call: the input view moves)
+    CUtensorMap tm[MAXL];               // per pyramid level: 3-D (x, y, frame) u8 tensor map with the 96x38 box of the stencil kernels
+                                        // (level 0 re-encoded per call: the input view moves)
     PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
     bool tma_levels_ok = false, use_tma = true;
-    bool use_pyr2 = false;              // SSLPL_PYR2=1: two levels per launch (k_pyr2); measured 1.00 ms against 0.85 ms for the seven k_resize launches (513 frames)
-    bool pyr2_ok[MAXL] = {};            // level pair (L, L+1) fits the tiles of k_pyr2 (checked against the resize tables)
     const uint8_t* tm0_base = nullptr; int tm0_pitch = 0, tm0_frames = 0; long long tm0_fs = 0;
 };
 
@@ -1022,18 +910,18 @@ int carve(sslpl_orb* h, Arena& A, const OrbGeom& g, int B, int W, int H) {
     ws.kps = A.take<sslpl_keypoint>((size_t)B * g.kp_total_cap);
     ws.desc = A.take<uint8_t>((size_t)B * g.kp_total_cap * 32);
     ws.nkp = A.take<int>(B);
-    ws.tmaps = A.take<CUtensorMap>(2 * MAXL);
+    ws.tmaps = A.take<CUtensorMap>(MAXL);
     return 0;
 }
 
-// 3-D u8 tensor map (x, y, frame) with an 80x38x1 box; returns false when the driver entry point is missing or the
+// 3-D u8 tensor map (x, y, frame) with a 96x38x1 box; returns false when the driver entry point is missing or the
 // view does not satisfy TMA's 16-byte alignment rules (then the kernels fall back to ordinary loads).
-bool encode_level_map(sslpl_orb* h, CUtensorMap* out, const uint8_t* base, int w, int hgt, int pitch, long long frame_stride, int frames, int bw = TL_P, int bh = TL_IH) {
+bool encode_level_map(sslpl_orb* h, CUtensorMap* out, const uint8_t* base, int w, int hgt, int pitch, long long frame_stride, int frames) {
     if (!h->encode) return false;
     if ((reinterpret_cast<uintptr_t>(base) & 15) || (pitch & 15) || (frame_stride & 15) || w < 1 || hgt < 1 || frames < 1) return false;
     const cuuint64_t gdim[3] = {(cuuint64_t)w, (cuuint64_t)hgt, (cuuint64_t)frames};
     const cuuint64_t gstr[2] = {(cuuint64_t)pitch, (cuuint64_t)frame_stride};
-    const cuuint32_t box[3] = {(cuuint32_t)bw, (cuuint32_t)bh, 1u};
+    const cuuint32_t box[3] = {(cuuint32_t)TL_P, (cuuint32_t)TL_IH, 1u};
     const cuuint32_t estr[3] = {1u, 1u, 1u};
     const CUresult r = h->encode(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<uint8_t*>(base), gdim, gstr, box, estr,
                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
@@ -1060,30 +948,8 @@ int configure(sslpl_orb* h, int W, int H) {
     h->tma_levels_ok = h->encode != nullptr;
     memset(&h->tm, 0, sizeof(h->tm));
     for (int l = 1; l < h->g.nlevels && h->tma_levels_ok; l++)
-        h->tma_levels_ok = encode_level_map(h, &h->tm.lvl[l], h->ws.pyr + h->g.lv[l].img_off, h->g.lv[l].w, h->g.lv[l].h, h->g.lv[l].pitch,
-                                            h->g.pyr_stride, h->p.max_batch) &&
-                           encode_level_map(h, &h->tm.pyr[l], h->ws.pyr + h->g.lv[l].img_off, h->g.lv[l].w, h->g.lv[l].h, h->g.lv[l].pitch,
-                                            h->g.pyr_stride, h->p.max_batch, PY_BW, PY_BH);
-    // which level pairs (L, L+1) can go through k_pyr2: every tile's spans in level L and level L-1 must fit its shared-memory tiles
-    for (int L = 1; L + 1 < h->g.nlevels; L++) {
-        const LevelGeom& S = h->g.lv[L - 1]; const LevelGeom& M = h->g.lv[L]; const LevelGeom& U = h->g.lv[L + 1];
-        bool ok = !rtab.empty();
-        auto span = [&](const int2* tU, const int2* tM, int un, int mn, int sn, int tile, int midcap, int boxcap, bool xaxis) {
-            for (int u0 = 0; u0 < un && ok; u0 += tile) {
-                const int u1 = std::min(u0 + tile, un);
-                const int c0 = tU[u0].x, c1 = u1 == un ? mn - 1 : std::min(tU[u1 - 1].x + 1, mn - 1);
-                const int q0 = xaxis ? (c0 & ~3) : c0;
-                if (c1 - q0 + 1 > midcap - (xaxis ? 3 : 0)) ok = false;
-                const int b0 = tM[c0].x, a0 = xaxis ? (b0 & ~15) : b0, b1 = std::min(tM[c1].x + 1, sn - 1);
-                if (b1 - a0 + 1 > boxcap) ok = false;
-            }
-        };
-        if (ok) {
-            span(rtab.data() + U.xtab_off, rtab.data() + M.xtab_off, U.w, M.w, S.w, PY_TW, PY_MP, PY_BW, true);
-            span(rtab.data() + U.ytab_off, rtab.data() + M.ytab_off, U.h, M.h, S.h, PY_TH, PY_MH, PY_BH, false);
-        }
-        h->pyr2_ok[L] = ok;
-    }
+        h->tma_levels_ok = encode_level_map(h, &h->tm[l], h->ws.pyr + h->g.lv[l].img_off, h->g.lv[l].w, h->g.lv[l].h, h->g.lv[l].pitch,
+                                            h->g.pyr_stride, h->p.max_batch);
     if (h->tma_levels_ok) SSLPL_CUDA(cudaMemcpy(h->ws.tmaps, &h->tm, sizeof(h->tm), cudaMemcpyHostToDevice));
     h->tm0_base = nullptr;
     h->cur_w = W; h->cur_h = H;
@@ -1106,25 +972,15 @@ int run_pipeline(sslpl_orb* h, int B) {
     bool tma = h->use_tma && h->tma_levels_ok;
     if (tma && !(h->tm0_base == h->view.base && h->tm0_pitch == h->view.pitch && h->tm0_fs == h->view.frame_stride && h->tm0_frames >= B)) {
         // level 0 is the caller's buffer: (re-)encode its maps when the view moves
-        tma = encode_level_map(h, &h->tm.lvl[0], h->view.base, g.lv[0].w, g.lv[0].h, h->view.pitch, h->view.frame_stride, B) &&
-              encode_level_map(h, &h->tm.pyr[0], h->view.base, g.lv[0].w, g.lv[0].h, h->view.pitch, h->view.frame_stride, B, PY_BW, PY_BH);
+        tma = encode_level_map(h, &h->tm[0], h->view.base, g.lv[0].w, g.lv[0].h, h->view.pitch, h->view.frame_stride, B);
         if (tma) {
-            SSLPL_CUDA(cudaMemcpyAsync(h->ws.tmaps, &h->tm.lvl[0], sizeof(CUtensorMap), cudaMemcpyHostToDevice, st));
-            SSLPL_CUDA(cudaMemcpyAsync(h->ws.tmaps + MAXL, &h->tm.pyr[0], sizeof(CUtensorMap), cudaMemcpyHostToDevice, st));
+            SSLPL_CUDA(cudaMemcpyAsync(h->ws.tmaps, &h->tm[0], sizeof(CUtensorMap), cudaMemcpyHostToDevice, st));
             h->tm0_base = h->view.base; h->tm0_pitch = h->view.pitch; h->tm0_fs = h->view.frame_stride; h->tm0_frames = B;
         } else h->tm0_base = nullptr;
     }
-    for (int l = 1; l < g.nlevels;) {
-        if (l + 1 < g.nlevels && h->pyr2_ok[l] && h->use_pyr2) {               // two levels per launch
-            const dim3 grid((g.lv[l + 1].w + PY_TW - 1) / PY_TW, (g.lv[l + 1].h + PY_TH - 1) / PY_TH, B);
-            if (tma) k_pyr2<true><<<grid, 256, 0, st>>>(g, h->ws, h->view, h->ws.tmaps, l);
-            else k_pyr2<false><<<grid, 256, 0, st>>>(g, h->ws, h->view, h->ws.tmaps, l);
-            l += 2;
-        } else {
-            dim3 grid((g.lv[l].w + 127) / 128, (g.lv[l].h + 7) / 8, B), block(32, 8);
-            k_resize<<<grid, block, 0, st>>>(g, h->ws, h->view, l);
-            l += 1;
-        }
+    for (int l = 1; l < g.nlevels; l++) {
+        dim3 grid((g.lv[l].w + 127) / 128, (g.lv[l].h + 7) / 8, B), block(32, 8);
+        k_resize<<<grid, block, 0, st>>>(g, h->ws, h->view, l);
         h->launches++;
     }
     mark(h, "pyramid");
@@ -1196,8 +1052,6 @@ int sslpl_orb_create(const sslpl_orb_params* p, sslpl_orb** out) {
         else cudaGetLastError();
         const char* e = getenv("SSLPL_NO_TMA");
         h->use_tma = !(e && e[0] == '1');
-        const char* e2 = getenv("SSLPL_PYR2");
-        h->use_pyr2 = e2 && e2[0] == '1';
     }
     *out = h;
     return SSLPL_OK;

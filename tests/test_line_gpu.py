@@ -117,28 +117,28 @@ def test_max_walkers_knob_does_not_change_results(pkg, synth):
         assert np.array_equal(got[3], ref[3]) and np.array_equal(got[1], ref[1]) and got[0].tobytes() == ref[0].tobytes(), cap
 
 
-WALKERS = [("one warp, round-2a form", {"SSLPL_WALKER_WARPS": "-1", "SSLPL_WALKER_LEAN": "0"}),
-           ("one warp, lean", {"SSLPL_WALKER_WARPS": "-1", "SSLPL_WALKER_LEAN": "1"}),
-           ("multi-warp round 2a, 16 warps", {"SSLPL_WALKER_WARPS": "16", "SSLPL_WALKER_V3": "0"}),
-           ("multi-warp round 2a, 5 warps", {"SSLPL_WALKER_WARPS": "5", "SSLPL_WALKER_V3": "0"}),
-           ("v3, 2 warps", {"SSLPL_WALKER_WARPS": "2", "SSLPL_WALKER_V3": "1"}),
-           ("v3, 3 warps", {"SSLPL_WALKER_WARPS": "3", "SSLPL_WALKER_V3": "1"}),
-           ("v3, 8 warps", {"SSLPL_WALKER_WARPS": "8", "SSLPL_WALKER_V3": "1"}),
-           ("v3, 16 warps", {"SSLPL_WALKER_WARPS": "16", "SSLPL_WALKER_V3": "1"}),
-           ("lane-parallel (experimental)", {"SSLPL_WALKER_WARPS": "-1", "SSLPL_WALKER_LANES": "1"})]
+WALKERS = [("one warp, round-2a form", {"SSLPL_WALKER_WARPS": "-1"}),
+           ("multi-warp round 2a, 16 warps", {"SSLPL_WALKER_WARPS": "16"}),
+           ("multi-warp round 2a, 5 warps", {"SSLPL_WALKER_WARPS": "5"}),
+           ("multi-warp round 2a, 2 warps", {"SSLPL_WALKER_WARPS": "2"}),
+           ("multi-warp round 2a, 3 warps", {"SSLPL_WALKER_WARPS": "3"}),
+           ("multi-warp round 2a, 4 warps", {"SSLPL_WALKER_WARPS": "4"}),
+           ("multi-warp round 2a, 8 warps", {"SSLPL_WALKER_WARPS": "8"}),
+           ("multi-warp round 2a, 12 warps", {"SSLPL_WALKER_WARPS": "12"}),
+           ("automatic choice", {})]
 
 
 @pytest.mark.parametrize("name,env", WALKERS, ids=[w[0] for w in WALKERS])
 def test_every_region_walker_is_the_sequential_one(pkg, oracle, synth, icl_gray, monkeypatch, name, env):
-    """The region stage exists in several forms (csrc/line.cu: one warp per frame in two forms, two multi-warp speculative walkers);
-    the handle picks one by batch and frame size.  Each of them, forced through the environment knobs that the handle reads when it
-    is created, has to reproduce the sequential detector: same raw segments, KeyLines and LBD bytes as the oracle, several runs each
-    (the multi-warp forms are timing dependent by construction)."""
-    for k in ("SSLPL_WALKER_WARPS", "SSLPL_WALKER_LEAN", "SSLPL_WALKER_V3", "SSLPL_WALKER_LANES"):
-        monkeypatch.delenv(k, raising=False)
+    """The region stage exists in two forms (csrc/line.cu: one warp per frame, k_lsd_regions_solo, and the multi-warp speculative
+    walker k_lsd_regions); the handle picks one by batch size.  Each of them, forced through SSLPL_WALKER_WARPS, which the handle
+    reads when it is created, at several warp counts, and the automatic choice (16 warps for these single frames), has to reproduce
+    the sequential detector: same raw segments, KeyLines and LBD bytes as the oracle, several runs each (the multi-warp form is
+    timing dependent by construction)."""
+    monkeypatch.delenv("SSLPL_WALKER_WARPS", raising=False)
     for k, v in env.items():
         monkeypatch.setenv(k, v)
-    reps = 1 if name.startswith("one warp") else (2 if name.startswith("lane") else 4)
+    reps = 1 if name.startswith("one warp") else 4
     for tag, img in (("icl", icl_gray), ("syn3", synth.frame(640, 480, 3)), ("syn8", synth.frame(640, 480, 8))):
         for _ in range(reps):
             _check_frame(pkg, oracle, img, 40, f"{name}/{tag}", vs_cv2=False)

@@ -120,12 +120,11 @@ def test_non_tma_fallback_path(pkg, oracle, synth, icl_gray, monkeypatch):
     _compare_all(ext2, oracle.OrbOracle(800, 1.2, 8, 20, 7), np.ascontiguousarray(img), "w613")
 
 
-def test_pyramid_two_levels_per_launch_path(pkg, oracle, synth, icl_gray, monkeypatch):
-    """SSLPL_PYR2=1 builds the pyramid two levels per launch (k_pyr2: level L-1 staged by TMA, level L recomputed with a halo in shared
-    memory) instead of one (k_resize, the default).  With and without TMA it must give the oracle's planes and keypoints — also at sizes
-    whose level widths are not multiples of the tiles."""
+def test_pyramid_odd_sizes(pkg, oracle, synth, icl_gray, monkeypatch):
+    """The pyramid (k_resize, one launch per level) and the TMA-staged kernels that read it must give the oracle's planes and
+    keypoints with and without TMA, also at sizes whose level widths are not multiples of the tiles."""
     orc = oracle.OrbOracle(1000, 1.2, 8, 20, 7)
-    for env in ({"SSLPL_PYR2": "1"}, {"SSLPL_PYR2": "1", "SSLPL_NO_TMA": "1"}, {}):
+    for env in ({}, {"SSLPL_NO_TMA": "1"}):
         for k, v in env.items():
             monkeypatch.setenv(k, v)
         ext = pkg.ORBextractor(1000, 1.2, 8, 20, 7, max_width=700, max_height=500)

@@ -17,25 +17,3 @@ def test_reduce_radius_compaction_matches_swap_with_last():
     import sim_reduce_radius as m
     assert m.run(iters=1500, seed=3)
 
-
-def test_lean_growth_lazy_angle_is_the_sequential_region_grow(tmp_path):
-    """Round 2b: the lean region growing (l_region_grow_lean, also the base of the v3 walker's growth) decides several neighbours per
-    round without recomputing the region angle when their outcome cannot change under a drift bound.  tools/sim_lean_grow.cpp runs the
-    warp algorithm lane by lane in lockstep with the oracle's sequential region_grow on real detection-scale frames (first growth and
-    refine's re-growth): every call must return the same list, in the same order, with the same angle."""
-    import subprocess
-    import numpy as np
-    sys.path.insert(0, ROOT)
-    import synth
-    from oracle import oracle as O
-    exe = str(tmp_path / "sim_lean_grow")
-    subprocess.run(["g++", "-O2", "-ffp-contract=off", "-I", os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tools", "sim_lean_grow.cpp"),
-                    os.path.join(ROOT, "oracle", "orb_oracle.cpp"), "-o", exe], check=True, capture_output=True)
-    for f, (w, h) in ((3, (640, 480)), (11, (320, 240))):
-        lo = O.LineOracle(40)
-        lo.extract(synth.frame(w, h, f))
-        sc = lo.scaled()
-        raw = tmp_path / f"s{f}.raw"
-        np.ascontiguousarray(sc).tofile(raw)
-        r = subprocess.run([exe, str(raw), str(sc.shape[1]), str(sc.shape[0])], capture_output=True, text=True)
-        assert r.returncode == 0 and " 0 mismatches" in r.stdout, r.stdout + r.stderr
