@@ -291,6 +291,43 @@ int  sslpl_match_bow_batch_device_vocab(sslpl_matcher* m, const uint8_t* d_desc,
 int  sslpl_match_lines_batch_device(sslpl_matcher* m, const uint8_t* d_ldesc, const int* d_nl, int nframes, int capl,
                                     int32_t* d_lmatch, int32_t* d_nlmatch);
 
+/* ---- Reference-keyframe matching of Tracking::TrackReferenceKeyFrame (Tracking.cc:1005-1034) against keyframes kept in HBM.
+   A keyframe set has max_keyframes slots on one device; a slot holds up to `cap` ORB descriptors with their keypoint angles and
+   MapPoint mask, their FeatureVector (built once, when the keyframe is stored), and up to `capl` LBD descriptors with their
+   MapLine mask.  Slots start empty; an empty or cleared slot matches nothing. ---- */
+typedef struct sslpl_kfset sslpl_kfset;
+int  sslpl_kfset_create(int device, int max_keyframes, int cap, int capl, sslpl_kfset** out);
+void sslpl_kfset_destroy(sslpl_kfset* k);
+/* Copy frame `frame` of an extraction batch's device results (d_desc/d_kps/d_n with `cap` rows per frame, d_ldesc/d_nl with `capl`)
+   into `slot` and build its FeatureVector with tree v at levelsup.  Masks are reset to all set.  Asynchronous on m's stream: the
+   caller orders it after the extraction, and the extractor's results may be overwritten once it has run. */
+int  sslpl_kfset_store_device(sslpl_matcher* m, sslpl_kfset* k, int slot,
+                              const uint8_t* d_desc, const sslpl_keypoint* d_kps, const int* d_n, int cap,
+                              const uint8_t* d_ldesc, const int* d_nl, int capl, int frame,
+                              const sslpl_vocab* v, int levelsup);
+/* The same from HOST buffers: n descriptors and keypoint angles, nl line descriptors.  Returns when the slot is written. */
+int  sslpl_kfset_store(sslpl_matcher* m, sslpl_kfset* k, int slot, const uint8_t* desc, const float* angle, int n,
+                       const uint8_t* ldesc, int nl, const sslpl_vocab* v, int levelsup);
+/* valid[i] != 0 <=> feature i holds a non-bad MapPoint; has_ml[j] != 0 <=> line j holds a MapLine (HOST buffers; NULL = all set;
+   entries past n / nl are set).  Returns when the masks are written, after the set's last store or match enqueued on a matcher's
+   stream (sslpl_kfset_clear too). */
+int  sslpl_kfset_set_masks(sslpl_kfset* k, int slot, const uint8_t* valid, int n, const uint8_t* has_ml, int nl);
+int  sslpl_kfset_clear(sslpl_kfset* k, int slot);
+/* For every frame f of a device extraction batch (layout as sslpl_match_bow_batch_device) with d_ref[f] = slot s (device int32
+   array, never read by the host; -1, or any value outside the set, = no reference keyframe):
+     ORBmatcher(nnratio, checkOrientation).SearchByBoW(KF s, frame f) (ORBmatcher.cc:159-291) with s's MapPoint mask:
+       d_match[f*cap + j] = KF feature index or -1, d_nmatch[f] = the reference's return value;
+     LSDmatcher::SearchByProjection(KF s, frame f) (LSDmatcher.cpp:143-183) with s's MapLine mask:
+       d_lmatch[f*capl + t] = KF line index or -1 (the last writer in KF line order), d_nlmatch[f] = the reference's return value
+       (0 when frame f has fewer than 2 lines, where the reference's knnMatch result is not usable).
+   Frames without a reference keyframe get -1 rows and 0 counts.  Every stored slot must have been built with v and levelsup
+   (SSLPL_ERR_ARG otherwise, nothing enqueued).  nframes <= max_batch + 1.  Asynchronous on m's stream. */
+int  sslpl_match_ref_kf_batch_device(sslpl_matcher* m, const sslpl_kfset* k, const int32_t* d_ref, int nframes,
+                                     const uint8_t* d_desc, const sslpl_keypoint* d_kps, const int* d_n, int cap,
+                                     const uint8_t* d_ldesc, const int* d_nl, int capl,
+                                     const sslpl_vocab* v, int levelsup, float nnratio, int checkOrientation,
+                                     int32_t* d_match, int32_t* d_nmatch, int32_t* d_lmatch, int32_t* d_nlmatch);
+
 /* =====================================================================================
  * (2) Line segments — replaces LineSegment::ExtractLineSegment (src/ExtractLineSegment.cpp:18-69)
  * ===================================================================================== */

@@ -446,6 +446,15 @@ class Matcher:
         _check(lib().sslpl_match_lines_batch_device(self._h, C.c_void_p(d_ldesc), C.c_void_p(d_nl), nframes, capl,
                                                     C.c_void_p(d_lmatch), C.c_void_p(d_nlmatch)))
 
+    def match_ref_kf_batch_device(self, kfset, d_ref, nframes, d_desc, d_kps, d_n, cap, d_ldesc, d_nl, capl, vocab, levelsup,
+                                  nnratio, check_ori, d_match, d_nmatch, d_lmatch, d_nlmatch):
+        """Tracking::TrackReferenceKeyFrame's two matchers for every frame f of a device batch against keyframe slot d_ref[f]
+        (-1 = none): SearchByBoW -> d_match[f, j] / d_nmatch[f], LSDmatcher::SearchByProjection -> d_lmatch[f, t] / d_nlmatch[f]."""
+        _check(lib().sslpl_match_ref_kf_batch_device(self._h, kfset._h, C.c_void_p(d_ref), nframes, C.c_void_p(d_desc), C.c_void_p(d_kps),
+                                                     C.c_void_p(d_n), cap, C.c_void_p(d_ldesc), C.c_void_p(d_nl), capl, vocab._h, int(levelsup),
+                                                     C.c_float(nnratio), int(check_ori), C.c_void_p(d_match), C.c_void_p(d_nmatch),
+                                                     C.c_void_p(d_lmatch), C.c_void_p(d_nlmatch)))
+
 
 class Vocabulary:
     """DBoW2 ORB vocabulary tree on the device (the reference's ORBVocabulary = TemplatedVocabulary<FORB::TDescriptor, FORB>,
@@ -555,6 +564,43 @@ class Vocabulary:
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
             lib().sslpl_vocab_destroy(self._h)
+            self._h = C.c_void_p()
+
+    __del__ = close
+
+
+class KeyframeSet:
+    """Reference keyframes kept in HBM for Matcher.match_ref_kf_batch_device (sslpl_kfset): max_keyframes slots of up to `cap`
+    features and `capl` lines each, with their FeatureVectors and MapPoint / MapLine masks."""
+
+    def __init__(self, max_keyframes, cap, capl, device=0):
+        self._h = C.c_void_p()
+        _check(lib().sslpl_kfset_create(device, max_keyframes, cap, capl, C.byref(self._h)))
+        self.max_keyframes, self.cap, self.capl = max_keyframes, cap, capl
+
+    def store_device(self, matcher, slot, d_desc, d_kps, d_n, cap, d_ldesc, d_nl, capl, frame, vocab, levelsup):
+        """Copy frame `frame` of an extraction batch's device results into `slot` (asynchronous on the matcher's stream)."""
+        _check(lib().sslpl_kfset_store_device(matcher._h, self._h, slot, C.c_void_p(d_desc), C.c_void_p(d_kps), C.c_void_p(d_n), cap,
+                                              C.c_void_p(d_ldesc), C.c_void_p(d_nl), capl, frame, vocab._h, int(levelsup)))
+
+    def store(self, matcher, slot, desc, angle, ldesc, vocab, levelsup):
+        desc = np.ascontiguousarray(desc, np.uint8).reshape(-1, 32); angle = np.ascontiguousarray(angle, np.float32)
+        ldesc = np.ascontiguousarray(ldesc, np.uint8).reshape(-1, 32)
+        assert len(angle) == len(desc)
+        _check(lib().sslpl_kfset_store(matcher._h, self._h, slot, _p(desc), _p(angle), len(desc), _p(ldesc), len(ldesc), vocab._h, int(levelsup)))
+
+    def set_masks(self, slot, valid=None, has_ml=None):
+        """valid[i] = feature i holds a non-bad MapPoint, has_ml[j] = line j holds a MapLine (None = all set)."""
+        v = np.ascontiguousarray(valid, np.uint8) if valid is not None else None
+        h = np.ascontiguousarray(has_ml, np.uint8) if has_ml is not None else None
+        _check(lib().sslpl_kfset_set_masks(self._h, slot, _p(v), 0 if v is None else len(v), _p(h), 0 if h is None else len(h)))
+
+    def clear(self, slot):
+        _check(lib().sslpl_kfset_clear(self._h, slot))
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            lib().sslpl_kfset_destroy(self._h)
             self._h = C.c_void_p()
 
     __del__ = close

@@ -4,7 +4,8 @@
 //
 // No tensor cores: 256-bit XOR + popcount per pair, reduced with warp shuffles.  Descriptors are read as
 // 2 x uint4 per row.  The batched layout is "a set of frames": frame f owns desc[f*cap..], a CSR feature
-// vector and optional masks; pair p matches frame p (KeyFrame role) against frame p+1 (Frame role).
+// vector and optional masks; pair p matches frame p (KeyFrame role) against frame p+1 (Frame role), or, for reference-keyframe
+// matching, frame f against the keyframe slot d_ref[f] of a keyframe set (sslpl_kfset).
 #include "common.cuh"
 #include <algorithm>
 #include <cmath>
@@ -40,15 +41,8 @@ __device__ __forceinline__ void top2_insert(unsigned& k0, unsigned& k1, unsigned
     if (k < k0) { k1 = k0; k0 = k; } else if (k < k1) k1 = k;
 }
 
-__global__ void __launch_bounds__(256) k_knn2(const uint8_t* q, long long q_fs, const int* nq_arr, int nq_const,
-                                               const uint8_t* t, long long t_fs, const int* nt_arr, int nt_const,
-                                               int32_t* out, long long out_fs, int qcap) {
-    const int pair = blockIdx.y, lane = threadIdx.x & 31, qi = blockIdx.x * 8 + (threadIdx.x >> 5);
-    const int nq = nq_arr ? min(nq_arr[pair], qcap) : nq_const, nt = nt_arr ? min(nt_arr[pair + 1], qcap) : nt_const;
-    if (qi >= nq) return;
-    uint4 a0, a1;
-    load_desc(q + pair * q_fs + (long long)qi * 32, a0, a1);
-    const uint8_t* T = t + pair * t_fs;
+// the two nearest of the nt train rows T to one query (a0, a1), computed by a whole warp; the result is in every lane
+__device__ __forceinline__ int4 knn2_warp(uint4 a0, uint4 a1, const uint8_t* T, int nt, int lane) {
     unsigned k0 = 0xffffffffu, k1 = 0xffffffffu;
     for (int j = lane; j < nt; j += 32) {
         uint4 b0, b1;
@@ -61,12 +55,22 @@ __global__ void __launch_bounds__(256) k_knn2(const uint8_t* q, long long q_fs, 
         top2_insert(k0, k1, o0);
         top2_insert(k0, k1, o1);
     }
-    if (lane == 0) {
-        int4 r;
-        r.x = k0 == 0xffffffffu ? -1 : (int)(k0 & 0xfffff); r.y = k0 == 0xffffffffu ? -1 : (int)(k0 >> 20);
-        r.z = k1 == 0xffffffffu ? -1 : (int)(k1 & 0xfffff); r.w = k1 == 0xffffffffu ? -1 : (int)(k1 >> 20);
-        reinterpret_cast<int4*>(out + pair * out_fs)[qi] = r;
-    }
+    int4 r;
+    r.x = k0 == 0xffffffffu ? -1 : (int)(k0 & 0xfffff); r.y = k0 == 0xffffffffu ? -1 : (int)(k0 >> 20);
+    r.z = k1 == 0xffffffffu ? -1 : (int)(k1 & 0xfffff); r.w = k1 == 0xffffffffu ? -1 : (int)(k1 >> 20);
+    return r;
+}
+
+__global__ void __launch_bounds__(256) k_knn2(const uint8_t* q, long long q_fs, const int* nq_arr, int nq_const,
+                                               const uint8_t* t, long long t_fs, const int* nt_arr, int nt_const,
+                                               int32_t* out, long long out_fs, int qcap) {
+    const int pair = blockIdx.y, lane = threadIdx.x & 31, qi = blockIdx.x * 8 + (threadIdx.x >> 5);
+    const int nq = nq_arr ? min(nq_arr[pair], qcap) : nq_const, nt = nt_arr ? min(nt_arr[pair + 1], qcap) : nt_const;
+    if (qi >= nq) return;
+    uint4 a0, a1;
+    load_desc(q + pair * q_fs + (long long)qi * 32, a0, a1);
+    const int4 r = knn2_warp(a0, a1, t + pair * t_fs, nt, lane);
+    if (lane == 0) reinterpret_cast<int4*>(out + pair * out_fs)[qi] = r;
 }
 
 // DescriptorDistance for n pairs (ORBmatcher.cc:1650): thread per pair
@@ -191,24 +195,11 @@ __device__ __forceinline__ int find_node(const int* nodes, int nn, int id) {   /
     return (lo < nn && nodes[lo] == id) ? lo : -1;
 }
 
-__global__ void __launch_bounds__(128) k_bow_match(FrameSet S, int mode, float nnratio, int cap,
-                                                    int32_t* out, long long out_fs, uint8_t* rot, long long rot_fs,
-                                                    uint8_t* taken, long long taken_fs) {
-    const int pair = blockIdx.y, lane = threadIdx.x & 31, a = blockIdx.x * 4 + (threadIdx.x >> 5);
-    const int f1 = pair, f2 = pair + 1;
-    const int nn1 = S.nn ? S.nn[f1] : S.nn_const, nn2 = S.nn ? S.nn[f2] : S.nn_const;
-    if (a >= nn1) return;
-    const int* nodes1 = S.nodes + f1 * S.nodes_fs; const int* nodes2 = S.nodes + f2 * S.nodes_fs;
-    const int b = find_node(nodes2, nn2, nodes1[a]);
-    if (b < 0) return;
-    const int* off1 = S.off + f1 * S.off_fs; const int* off2 = S.off + f2 * S.off_fs;
-    const int* idx1 = S.idx + f1 * S.idx_fs; const int* idx2 = S.idx + f2 * S.idx_fs;
-    const uint8_t* D1 = S.desc + f1 * S.desc_fs; const uint8_t* D2 = S.desc + f2 * S.desc_fs;
-    const uint8_t* v1 = S.flag ? S.flag + f1 * S.flag_fs : nullptr;
-    const uint8_t* v2 = S.flag ? S.flag + f2 * S.flag_fs : nullptr;
-    const float* A1 = S.angle + f1 * S.angle_fs; const float* A2 = S.angle + f2 * S.angle_fs;
-    int32_t* O = out + pair * out_fs; uint8_t* R = rot + pair * rot_fs; uint8_t* TK = taken + pair * taken_fs;
-    const int b1 = off1[a], e1 = off1[a + 1], b2 = off2[b], e2 = off2[b + 1];
+// One node shared by both FeatureVectors: KF features idx1[b1..e1) against frame features idx2[b2..e2), in list order.
+__device__ __forceinline__ void bow_match_node(int mode, float nnratio, int lane, int b1, int e1, int b2, int e2,
+                                               const int* idx1, const int* idx2, const uint8_t* D1, const uint8_t* D2,
+                                               const uint8_t* v1, const uint8_t* v2, const float* A1, int es1, const float* A2, int es2,
+                                               int32_t* O, uint8_t* R, uint8_t* TK) {
     for (int i1 = b1; i1 < e1; i1++) {
         const int id1 = idx1[i1];
         if (v1 && !v1[id1]) continue;                                            // :196-200 / :563-567
@@ -238,13 +229,108 @@ __global__ void __launch_bounds__(128) k_bow_match(FrameSet S, int mode, float n
             const int id2 = idx2[b2 + (int)(k0 & 0xfffff)];
             if (lane == 0) {
                 TK[id2] = 1;
-                const int bin = rot_bin(A1[(long long)id1 * S.angle_es], A2[(long long)id2 * S.angle_es]);
+                const int bin = rot_bin(A1[(long long)id1 * es1], A2[(long long)id2 * es2]);
                 if (mode == 0) { O[id2] = id1; R[id2] = (uint8_t)bin; }
                 else { O[id1] = id2; R[id1] = (uint8_t)bin; }
             }
         }
         __syncwarp();
     }
+}
+
+__global__ void __launch_bounds__(128) k_bow_match(FrameSet S, int mode, float nnratio, int cap,
+                                                    int32_t* out, long long out_fs, uint8_t* rot, long long rot_fs,
+                                                    uint8_t* taken, long long taken_fs) {
+    const int pair = blockIdx.y, lane = threadIdx.x & 31, a = blockIdx.x * 4 + (threadIdx.x >> 5);
+    const int f1 = pair, f2 = pair + 1;
+    const int nn1 = S.nn ? S.nn[f1] : S.nn_const, nn2 = S.nn ? S.nn[f2] : S.nn_const;
+    if (a >= nn1) return;
+    const int* nodes1 = S.nodes + f1 * S.nodes_fs; const int* nodes2 = S.nodes + f2 * S.nodes_fs;
+    const int b = find_node(nodes2, nn2, nodes1[a]);
+    if (b < 0) return;
+    const int* off1 = S.off + f1 * S.off_fs; const int* off2 = S.off + f2 * S.off_fs;
+    const int* idx1 = S.idx + f1 * S.idx_fs; const int* idx2 = S.idx + f2 * S.idx_fs;
+    const uint8_t* D1 = S.desc + f1 * S.desc_fs; const uint8_t* D2 = S.desc + f2 * S.desc_fs;
+    const uint8_t* v1 = S.flag ? S.flag + f1 * S.flag_fs : nullptr;
+    const uint8_t* v2 = S.flag ? S.flag + f2 * S.flag_fs : nullptr;
+    const float* A1 = S.angle + f1 * S.angle_fs; const float* A2 = S.angle + f2 * S.angle_fs;
+    int32_t* O = out + pair * out_fs; uint8_t* R = rot + pair * rot_fs; uint8_t* TK = taken + pair * taken_fs;
+    bow_match_node(mode, nnratio, lane, off1[a], off1[a + 1], off2[b], off2[b + 1], idx1, idx2, D1, D2, v1, v2,
+                   A1, S.angle_es, A2, S.angle_es, O, R, TK);
+}
+
+// -------------------------------------------------------------------------------------------------
+// Keyframe set (sslpl_kfset): per slot s, `cap` ORB rows and `capl` LBD rows.  The FeatureVector is sparse: nn[s] non-empty
+// nodes in ascending id, nodes[s*cap + a], off[s*(cap+1) + a], idx[s*cap + ..] (a node holds at least one feature, so
+// nn <= cap).  An empty or cleared slot has nn = n = nl = 0 and matches nothing.
+// -------------------------------------------------------------------------------------------------
+struct KfView {
+    uint8_t* desc; float* angle; uint8_t* valid;
+    int* nodes; int* off; int* idx; int* nn;
+    uint8_t* ldesc; uint8_t* has_ml; int* nl;
+    int cap, capl, nslots;
+};
+
+__device__ __forceinline__ int kf_slot(const KfView& K, const int32_t* ref, int f) {
+    const int s = ref[f];
+    return (s >= 0 && s < K.nslots) ? s : -1;
+}
+
+// Keyframe side of a stored slot's FeatureVector: k_build_csr's dense offsets (nc + 1 entries) compacted to the non-empty
+// nodes, and the slot's line count.  One CTA of 256 threads.
+__global__ void __launch_bounds__(256) k_kf_compact(const int* dense_off, int nc, const int* nl_src, int capl_src,
+                                                     int* nodes, int* off, int* nn, int* nl_out) {
+    __shared__ int s_warp[33];
+    int base = 0;
+    for (int c0 = 0; c0 < nc; c0 += 256) {
+        const int c = c0 + threadIdx.x;
+        const int lo = c < nc ? dense_off[c] : 0;
+        const int keep = c < nc && dense_off[c + 1] > lo;
+        int total;
+        const int o = base + block_exclusive_scan(keep, s_warp, &total);
+        if (keep) { nodes[o] = c; off[o] = lo; }
+        base += total;
+    }
+    if (threadIdx.x == 0) {
+        off[base] = dense_off[nc];
+        *nn = base;
+        *nl_out = min(*nl_src, capl_src);
+    }
+}
+
+// SearchByBoW(KF ref[f], frame f), mode 0 (ORBmatcher.cc:159-291): one warp per (frame, node of the keyframe).  The frame side
+// is the batch's dense FeatureVector (S.nodes = 0..nc-1).
+__global__ void __launch_bounds__(128) k_bow_match_ref(KfView K, const int32_t* ref, FrameSet S, float nnratio,
+                                                        int32_t* out, long long out_fs, uint8_t* rot, long long rot_fs,
+                                                        uint8_t* taken, long long taken_fs) {
+    const int f = blockIdx.y, lane = threadIdx.x & 31, a = blockIdx.x * 4 + (threadIdx.x >> 5);
+    const int s = kf_slot(K, ref, f);
+    if (s < 0 || a >= K.nn[s]) return;
+    const long long ks = (long long)s * K.cap;
+    const int b = find_node(S.nodes, S.nn_const, K.nodes[ks + a]);
+    if (b < 0) return;
+    const int* off1 = K.off + (long long)s * (K.cap + 1); const int* off2 = S.off + f * S.off_fs;
+    bow_match_node(0, nnratio, lane, off1[a], off1[a + 1], off2[b], off2[b + 1], K.idx + ks, S.idx + f * S.idx_fs,
+                   K.desc + ks * 32, S.desc + f * S.desc_fs, K.valid + ks, nullptr, K.angle + ks, 1, S.angle + f * S.angle_fs, S.angle_es,
+                   out + f * out_fs, rot + f * rot_fs, taken + f * taken_fs);
+}
+
+// knnMatch(KF ref[f] lines, frame f lines, k=2) for LSDmatcher::SearchByProjection(KF,F) (LSDmatcher.cpp:155): row q of frame f
+// is the KF line q's two nearest frame lines, or -1s when the slot is empty, q is past its lines, or line q holds no MapLine
+// (:169 rejects those rows whatever their distances), so k_line_ratio needs no mask.  Rows [0, qcap) are all written.
+__global__ void __launch_bounds__(256) k_knn2_ref(KfView K, const int32_t* ref, const uint8_t* t, long long t_fs, const int* nt_arr, int ntcap,
+                                                   int32_t* out, long long out_fs, int qcap) {
+    const int f = blockIdx.y, lane = threadIdx.x & 31, qi = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (qi >= qcap) return;
+    const int s = kf_slot(K, ref, f);
+    const long long ks = (long long)max(s, 0) * K.capl;
+    int4 r = make_int4(-1, -1, -1, -1);
+    if (s >= 0 && qi < K.nl[s] && K.has_ml[ks + qi]) {
+        uint4 a0, a1;
+        load_desc(K.ldesc + (ks + qi) * 32, a0, a1);
+        r = knn2_warp(a0, a1, t + f * t_fs, min(nt_arr[f], ntcap), lane);
+    }
+    if (lane == 0) reinterpret_cast<int4*>(out + f * out_fs)[qi] = r;
 }
 
 // SearchForTriangulation (ORBmatcher.cc:660-826, monocular): warp per node of set 1; no dependency between
@@ -910,6 +996,16 @@ struct sslpl_matcher {
     int32_t* b_node; int* b_off; int* b_idx; uint8_t* b_rot; uint8_t* b_taken; int32_t* b_knn; int* iota;
     int32_t* h_small = nullptr;      // pinned scratch
     long long launches = 0;
+};
+
+struct sslpl_kfset {
+    int device = 0;
+    sslpl::KfView view{};            // device arrays of every slot (layout above k_kf_compact)
+    uint8_t* arena = nullptr;
+    cudaStream_t stream = nullptr;   // host-buffer mask uploads and clears
+    cudaEvent_t last_use = nullptr;  // recorded after every store / match enqueued on a matcher's stream
+    struct Built { const sslpl_vocab* v; int levelsup; };
+    std::vector<Built> built;        // tree and levelsup of each slot's FeatureVector; v == nullptr: empty slot
 };
 
 namespace {
@@ -1793,6 +1889,189 @@ int sslpl_match_lines_batch_device(sslpl_matcher* m, const uint8_t* d_ldesc, con
     k_line_ratio<<<dim3((capl + 127) / 128, npairs), 128, 0, st>>>(m->b_knn, (long long)lc * 4, d_nl, 0, capl, nullptr, 0, d_lmatch, capl, d_nlmatch);
     m->launches++;
     SSLPL_CUDA(cudaGetLastError());
+    return SSLPL_OK;
+}
+
+// ---------------- keyframe set and reference-keyframe matching (Tracking::TrackReferenceKeyFrame, Tracking.cc:1005-1034) ----------------
+void sslpl_kfset_destroy(sslpl_kfset* k);
+
+int sslpl_kfset_create(int device, int max_keyframes, int cap, int capl, sslpl_kfset** out) {
+    SSLPL_REQUIRE(out, SSLPL_ERR_ARG, "null argument");
+    SSLPL_REQUIRE(max_keyframes >= 1 && cap >= 1 && capl >= 1 && cap < (1 << 20) && capl < (1 << 20), SSLPL_ERR_ARG, "bad keyframe set capacity");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) { set_error("no CUDA device available: libsslpl_b200 has no CPU fallback"); return SSLPL_ERR_CUDA; }
+    SSLPL_CUDA(cudaSetDevice(device));
+    const size_t K = max_keyframes;
+    auto carve_all = [&](Arena& a, KfView& w) {
+        w.desc = a.take<uint8_t>(K * cap * 32); w.angle = a.take<float>(K * cap); w.valid = a.take<uint8_t>(K * cap);
+        w.nodes = a.take<int>(K * cap); w.off = a.take<int>(K * (cap + 1)); w.idx = a.take<int>(K * cap); w.nn = a.take<int>(K);
+        w.ldesc = a.take<uint8_t>(K * capl * 32); w.has_ml = a.take<uint8_t>(K * capl); w.nl = a.take<int>(K);
+    };
+    Arena A; KfView dry{}; carve_all(A, dry);
+    sslpl_kfset* k = new sslpl_kfset();
+    k->device = device;
+    k->built.assign(K, {nullptr, 0});
+    cudaError_t e = cudaMalloc(&k->arena, A.used + 256);
+    if (e != cudaSuccess) { set_error("cudaMalloc(%zu) failed: %s", A.used + 256, cudaGetErrorString(e)); delete k; return SSLPL_ERR_CUDA; }
+    Arena B; B.base = k->arena; carve_all(B, k->view);
+    k->view.cap = cap; k->view.capl = capl; k->view.nslots = max_keyframes;
+    e = cudaMemset(k->arena, 0, A.used + 256);                      // every slot empty: nn = n = nl = 0
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&k->stream, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&k->last_use, cudaEventDisableTiming);
+    if (e != cudaSuccess) { set_error("sslpl_kfset_create: %s", cudaGetErrorString(e)); sslpl_kfset_destroy(k); return SSLPL_ERR_CUDA; }
+    *out = k;
+    return SSLPL_OK;
+}
+
+void sslpl_kfset_destroy(sslpl_kfset* k) {
+    if (!k) return;
+    cudaSetDevice(k->device);
+    if (k->last_use) { cudaEventSynchronize(k->last_use); cudaEventDestroy(k->last_use); }
+    if (k->stream) { cudaStreamSynchronize(k->stream); cudaStreamDestroy(k->stream); }
+    if (k->arena) cudaFree(k->arena);
+    delete k;
+}
+
+// FeatureVector and counts of slot `slot`, whose descriptors are already (being) copied in, from n_src / nl_src (device)
+static int kf_index(sslpl_matcher* m, sslpl_kfset* k, int slot, const int* n_src, int cap_src, const int* nl_src, int capl_src,
+                    const sslpl_vocab* v, int levelsup) {
+    cudaStream_t st = m->stream;
+    const KfView& K = k->view;
+    const long long ks = (long long)slot * K.cap;
+    const int nc = vocab_level_nodes(v, levelsup);
+    k_vocab_transform<<<dim3((cap_src + 127) / 128, 1), 128, 0, st>>>(K.desc + ks * 32, 0, n_src, 0, cap_src, v->view, v->L - levelsup,
+                                                                       nullptr, nullptr, m->b_node, nullptr, 0);
+    k_build_csr<<<1, 128, (nc + 1 + cap_src) * sizeof(int), st>>>(m->b_node, 0, n_src, cap_src, nc, m->b_off, 0, K.idx + ks, 0);
+    k_kf_compact<<<1, 256, 0, st>>>(m->b_off, nc, nl_src, capl_src, K.nodes + ks, K.off + (long long)slot * (K.cap + 1), K.nn + slot, K.nl + slot);
+    m->launches += 3;
+    SSLPL_CUDA(cudaGetLastError());
+    SSLPL_CUDA(cudaMemsetAsync(K.valid + ks, 1, K.cap, st));
+    SSLPL_CUDA(cudaMemsetAsync(K.has_ml + (long long)slot * K.capl, 1, K.capl, st));
+    SSLPL_CUDA(cudaEventRecord(k->last_use, st));
+    k->built[slot] = {v, levelsup};
+    return SSLPL_OK;
+}
+
+static int kf_store_checks(sslpl_matcher* m, sslpl_kfset* k, int slot, int cap, int capl, const sslpl_vocab* v, int levelsup) {
+    SSLPL_REQUIRE(m && k && v, SSLPL_ERR_ARG, "null argument");
+    SSLPL_REQUIRE(slot >= 0 && slot < k->view.nslots, SSLPL_ERR_ARG, "slot outside the keyframe set");
+    SSLPL_REQUIRE(cap >= 0 && cap <= k->view.cap && cap <= m->p.max_features + 64, SSLPL_ERR_ARG, "cap exceeds the keyframe set or the matcher capacity");
+    SSLPL_REQUIRE(capl >= 0 && capl <= k->view.capl, SSLPL_ERR_ARG, "capl exceeds the keyframe set capacity");
+    SSLPL_REQUIRE(k->device == m->p.device && v->device == m->p.device, SSLPL_ERR_ARG, "keyframe set, vocabulary and matcher live on different devices");
+    const int nc = vocab_level_nodes(v, levelsup);
+    SSLPL_REQUIRE(nc <= m->p.max_nodes, SSLPL_ERR_ARG, "the vocabulary level exceeds the matcher capacity (max_nodes)");
+    SSLPL_REQUIRE((size_t)((nc + 1 + cap) * sizeof(int)) <= (size_t)MAX_DYN_SMEM, SSLPL_ERR_CAPACITY, "nodes + features exceed the shared memory of one CTA ((nc + 1 + cap) * 4 <= 200 KB)");
+    return SSLPL_OK;
+}
+
+int sslpl_kfset_store_device(sslpl_matcher* m, sslpl_kfset* k, int slot,
+                             const uint8_t* d_desc, const sslpl_keypoint* d_kps, const int* d_n, int cap,
+                             const uint8_t* d_ldesc, const int* d_nl, int capl, int frame,
+                             const sslpl_vocab* v, int levelsup) {
+    if (int rc = kf_store_checks(m, k, slot, cap, capl, v, levelsup)) return rc;
+    SSLPL_REQUIRE(d_desc && d_kps && d_n && d_ldesc && d_nl && cap >= 1 && capl >= 1 && frame >= 0, SSLPL_ERR_ARG, "null argument or empty frame capacity");
+    SSLPL_CUDA(cudaSetDevice(m->p.device));
+    cudaStream_t st = m->stream;
+    const KfView& K = k->view;
+    const long long ks = (long long)slot * K.cap, f = frame;
+    SSLPL_CUDA(cudaMemcpyAsync(K.desc + ks * 32, d_desc + f * cap * 32, (size_t)cap * 32, cudaMemcpyDeviceToDevice, st));
+    SSLPL_CUDA(cudaMemcpy2DAsync(K.angle + ks, sizeof(float), reinterpret_cast<const float*>(d_kps + f * cap) + 3,
+                                 sizeof(sslpl_keypoint), sizeof(float), cap, cudaMemcpyDeviceToDevice, st));
+    SSLPL_CUDA(cudaMemcpyAsync(K.ldesc + (long long)slot * K.capl * 32, d_ldesc + f * capl * 32, (size_t)capl * 32,
+                               cudaMemcpyDeviceToDevice, st));
+    return kf_index(m, k, slot, d_n + frame, cap, d_nl + frame, capl, v, levelsup);
+}
+
+int sslpl_kfset_store(sslpl_matcher* m, sslpl_kfset* k, int slot, const uint8_t* desc, const float* angle, int n,
+                      const uint8_t* ldesc, int nl, const sslpl_vocab* v, int levelsup) {
+    if (int rc = kf_store_checks(m, k, slot, n, nl, v, levelsup)) return rc;
+    SSLPL_REQUIRE((n == 0 || (desc && angle)) && (nl == 0 || ldesc), SSLPL_ERR_ARG, "null descriptor / angle array");
+    SSLPL_CUDA(cudaSetDevice(m->p.device));
+    cudaStream_t st = m->stream;
+    const KfView& K = k->view;
+    const long long ks = (long long)slot * K.cap;
+    if (n) SSLPL_CUDA(cudaMemcpyAsync(K.desc + ks * 32, desc, (size_t)n * 32, cudaMemcpyHostToDevice, st));
+    if (n) SSLPL_CUDA(cudaMemcpyAsync(K.angle + ks, angle, sizeof(float) * n, cudaMemcpyHostToDevice, st));
+    if (nl) SSLPL_CUDA(cudaMemcpyAsync(K.ldesc + (long long)slot * K.capl * 32, ldesc, (size_t)nl * 32, cudaMemcpyHostToDevice, st));
+    m->h_small[0] = n; m->h_small[1] = nl;
+    SSLPL_CUDA(cudaMemcpyAsync(m->ncnt, m->h_small, 2 * sizeof(int), cudaMemcpyHostToDevice, st));
+    if (int rc = kf_index(m, k, slot, m->ncnt, std::max(n, 1), m->ncnt + 1, std::max(nl, 1), v, levelsup)) return rc;
+    SSLPL_CUDA(cudaStreamSynchronize(st));                                // the caller's host buffers and h_small are free again
+    return SSLPL_OK;
+}
+
+int sslpl_kfset_set_masks(sslpl_kfset* k, int slot, const uint8_t* valid, int n, const uint8_t* has_ml, int nl) {
+    SSLPL_REQUIRE(k, SSLPL_ERR_ARG, "null argument");
+    SSLPL_REQUIRE(slot >= 0 && slot < k->view.nslots, SSLPL_ERR_ARG, "slot outside the keyframe set");
+    SSLPL_REQUIRE(n >= 0 && n <= k->view.cap && nl >= 0 && nl <= k->view.capl, SSLPL_ERR_ARG, "mask longer than the keyframe set capacity");
+    SSLPL_CUDA(cudaSetDevice(k->device));
+    const KfView& K = k->view;
+    uint8_t* mv = K.valid + (long long)slot * K.cap;
+    uint8_t* ml = K.has_ml + (long long)slot * K.capl;
+    SSLPL_CUDA(cudaStreamWaitEvent(k->stream, k->last_use, 0));          // after the store that reset them and the matches that read them
+    SSLPL_CUDA(cudaMemsetAsync(mv, 1, K.cap, k->stream));
+    if (valid && n) SSLPL_CUDA(cudaMemcpyAsync(mv, valid, n, cudaMemcpyHostToDevice, k->stream));
+    SSLPL_CUDA(cudaMemsetAsync(ml, 1, K.capl, k->stream));
+    if (has_ml && nl) SSLPL_CUDA(cudaMemcpyAsync(ml, has_ml, nl, cudaMemcpyHostToDevice, k->stream));
+    SSLPL_CUDA(cudaStreamSynchronize(k->stream));
+    return SSLPL_OK;
+}
+
+int sslpl_kfset_clear(sslpl_kfset* k, int slot) {
+    SSLPL_REQUIRE(k, SSLPL_ERR_ARG, "null argument");
+    SSLPL_REQUIRE(slot >= 0 && slot < k->view.nslots, SSLPL_ERR_ARG, "slot outside the keyframe set");
+    SSLPL_CUDA(cudaSetDevice(k->device));
+    SSLPL_CUDA(cudaStreamWaitEvent(k->stream, k->last_use, 0));
+    SSLPL_CUDA(cudaMemsetAsync(k->view.nn + slot, 0, sizeof(int), k->stream));
+    SSLPL_CUDA(cudaMemsetAsync(k->view.nl + slot, 0, sizeof(int), k->stream));
+    SSLPL_CUDA(cudaStreamSynchronize(k->stream));
+    k->built[slot] = {nullptr, 0};
+    return SSLPL_OK;
+}
+
+int sslpl_match_ref_kf_batch_device(sslpl_matcher* m, const sslpl_kfset* k, const int32_t* d_ref, int nframes,
+                                    const uint8_t* d_desc, const sslpl_keypoint* d_kps, const int* d_n, int cap,
+                                    const uint8_t* d_ldesc, const int* d_nl, int capl,
+                                    const sslpl_vocab* v, int levelsup, float nnratio, int checkOri,
+                                    int32_t* d_match, int32_t* d_nmatch, int32_t* d_lmatch, int32_t* d_nlmatch) {
+    SSLPL_REQUIRE(m && k && v && d_ref && d_desc && d_kps && d_n && d_ldesc && d_nl && d_match && d_nmatch && d_lmatch && d_nlmatch,
+                  SSLPL_ERR_ARG, "null argument");
+    SSLPL_REQUIRE(nframes >= 1 && nframes <= m->p.max_batch + 1, SSLPL_ERR_ARG, "nframes exceeds max_batch+1");
+    const int fc = m->p.max_features + 64, lc = m->p.max_lines + 64, NN = m->p.max_nodes + 1;
+    SSLPL_REQUIRE(cap >= 1 && cap <= fc && capl >= 1 && capl <= lc, SSLPL_ERR_ARG, "cap or capl exceeds the matcher capacity");
+    SSLPL_REQUIRE(k->view.capl <= lc, SSLPL_ERR_ARG, "the keyframe set holds more lines per keyframe than the matcher's max_lines + 64");
+    SSLPL_REQUIRE(k->device == m->p.device && v->device == m->p.device, SSLPL_ERR_ARG, "keyframe set, vocabulary and matcher live on different devices");
+    const int nc = vocab_level_nodes(v, levelsup);
+    SSLPL_REQUIRE(nc <= m->p.max_nodes, SSLPL_ERR_ARG, "the vocabulary level exceeds the matcher capacity (max_nodes)");
+    for (const auto& b : k->built)
+        SSLPL_REQUIRE(!b.v || (b.v == v && b.levelsup == levelsup), SSLPL_ERR_ARG, "a stored keyframe was built with another vocabulary tree or levelsup");
+    SSLPL_REQUIRE((size_t)((nc + 1 + cap) * sizeof(int)) <= (size_t)MAX_DYN_SMEM, SSLPL_ERR_CAPACITY, "nodes + features exceed the shared memory of one CTA ((nc + 1 + cap) * 4 <= 200 KB)");
+    SSLPL_CUDA(cudaSetDevice(m->p.device));
+    cudaStream_t st = m->stream;
+    // points: the batch's dense FeatureVectors (as sslpl_match_bow_batch_device_vocab), then SearchByBoW against the slots
+    k_vocab_transform<<<dim3((cap + 127) / 128, nframes), 128, 0, st>>>(d_desc, (long long)cap * 32, d_n, 0, cap, v->view, v->L - levelsup,
+                                                                         nullptr, nullptr, m->b_node, nullptr, fc);
+    k_build_csr<<<nframes, 128, (nc + 1 + cap) * sizeof(int), st>>>(m->b_node, fc, d_n, cap, nc, m->b_off, NN + 1, m->b_idx, fc);
+    m->launches += 2;
+    fill(m, d_match, (long long)nframes * cap, -1);
+    SSLPL_CUDA(cudaMemsetAsync(m->b_rot, 255, (size_t)nframes * fc, st));
+    SSLPL_CUDA(cudaMemsetAsync(m->b_taken, 0, (size_t)nframes * fc, st));
+    FrameSet S; memset(&S, 0, sizeof(S));
+    S.desc = d_desc; S.desc_fs = (long long)cap * 32;
+    S.nodes = m->iota; S.nn_const = nc; S.off = m->b_off; S.idx = m->b_idx; S.off_fs = NN + 1; S.idx_fs = fc;
+    S.angle = reinterpret_cast<const float*>(d_kps) + 3; S.angle_es = 7; S.angle_fs = (long long)cap * 7;
+    k_bow_match_ref<<<dim3((std::min(k->view.cap, nc) + 3) / 4, nframes), 128, 0, st>>>(k->view, d_ref, S, nnratio, d_match, cap, m->b_rot, fc,
+                                                                                          m->b_taken, fc);
+    k_rot_filter<<<nframes, 256, 0, st>>>(d_match, cap, m->b_rot, fc, d_n, 0, 0, cap, checkOri, d_nmatch, nullptr, 0);
+    // lines: knn2 of the slot's MapLine-holding lines against frame f's, then the ratio rule
+    const int qcap = k->view.capl;
+    k_knn2_ref<<<dim3((qcap + 7) / 8, nframes), 256, 0, st>>>(k->view, d_ref, d_ldesc, (long long)capl * 32, d_nl, capl, m->b_knn, (long long)lc * 4, qcap);
+    fill(m, d_lmatch, (long long)nframes * capl, -1);
+    SSLPL_CUDA(cudaMemsetAsync(d_nlmatch, 0, sizeof(int32_t) * nframes, st));
+    k_line_ratio<<<dim3((qcap + 127) / 128, nframes), 128, 0, st>>>(m->b_knn, (long long)lc * 4, nullptr, qcap, qcap, nullptr, 0, d_lmatch, capl, d_nlmatch);
+    m->launches += 4;
+    SSLPL_CUDA(cudaGetLastError());
+    SSLPL_CUDA(cudaEventRecord(k->last_use, st));
     return SSLPL_OK;
 }
 
